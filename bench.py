@@ -6,6 +6,8 @@ DOF-timesteps/s; assembly cells/s and nnz/s are reported beside it).
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the reference's solver configuration
                                                            # restated in C + OpenMP on all host cores
                                                            # (DOLFINx/PETSc cannot be installed)
+  python bench.py --gpus 1 ... --dump-outputs DIR          # also writes the solution of the last timed step
+                                                           # as DIR/velocity.npy and DIR/pressure.npy
 
 A "step" is one time step (`Solver.solveStep`) of the workload: Newton with Jacobian + residual assemblies and a
 preconditioned FGMRES solve per iteration.  `value` is measured with everything resident in HBM
@@ -69,6 +71,7 @@ DEFAULT_WORKLOAD = "lid_driven2D_nx512"
 EXTRA_WORKLOADS = [("lid_driven2D_nx707", 3, 10), ("stenosis_pressure_structured_16m", 2, 4)]
 CPU_BUDGET_S = 1500.0        # the CPU arm stops taking new steps beyond this (driver limit: 1800 s per arm)
 CPU_BUDGET_WEAK_S = 420.0    # the same for the weak-scaled meshes of the N > 1 lines (minutes per time step)
+DUMP_BYTES = 64_000_000      # --dump-outputs writes at most this many bytes of array data
 
 PROF_CLASSES = {0: "spmv_node(J)", 1: "cell_jacobian", 2: "gather_matrix", 3: "cell_residual",
                 4: "cheb_step<2>(A00,l0)", 5: "cheb_step<1>(Lp,l0)", 6: "mdot", 7: "maxpy_norm",
@@ -128,6 +131,19 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as dirname/<name>.npy in float64.  When they hold more than DUMP_BYTES in all, each is cut to
+    a fixed, seeded sample of its entries (in index order), the same from run to run for the same workload."""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(8 * a.size for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).reshape(-1)
+        if total > DUMP_BYTES:
+            keep = np.random.default_rng(0).choice(a.size, a.size * DUMP_BYTES // total, replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def build_scenario(w, **solver_kw):
@@ -209,7 +225,7 @@ def run_reference(args):
                          "(asm/ilu(0) sub-solves, stabilized_schur.py:256-267) and stenosis_pressure_structured (lu sub-solves, "
                          "stabilized_schur_pressure_backflow.py:284-288) workloads")
     W = max(0, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
     N = max(int(args.gpus), 1)
     nx = None
     budget = CPU_BUDGET_S
@@ -280,7 +296,7 @@ def hierarchy_bytes(s):
     return out
 
 
-def measure_workload(name, W, K, local_rank, want_e2e=True, want_prof=True, solver_kw=None):
+def measure_workload(name, W, K, local_rank, want_e2e=True, want_prof=True, solver_kw=None, dump_dir=None):
     import torch
     w = WORKLOADS[name]
     t_build = time.perf_counter()
@@ -317,6 +333,9 @@ def measure_workload(name, W, K, local_rank, want_e2e=True, want_prof=True, solv
     ms = e0.elapsed_time(e1)
     launches = hemo.launches - launches0
     clocks = sampler.stop()
+    if dump_dir:
+        # the solution of the last timed step, as step_device() leaves it for its caller (the steps below march on)
+        dump_outputs(dump_dir, {"velocity": s.d_x[:2 * n].cpu().numpy(), "pressure": s.d_x[2 * n:].cpu().numpy()})
     out = dict(config=workload_config(name, sc), value=ndof * K / (ms * 1e-3), ms_per_step=ms / K, steps=K, warmup=W,
                newton_its_per_step=newton / K, fgmres_its_per_step=ksp / K, gpu_launches=launches, clocks=clocks,
                nnz=nnz, build_s=t_build)
@@ -591,7 +610,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the larger GPU-only workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the velocity and pressure of the last timed step as DIR/<name>.npy (float64, at most "
+                         "64 MB in all; a fixed, seeded sample of larger solutions); single-GPU arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU arm only")
     _guard_stdout()
     if args.impl == "reference":
         run_reference(args)
@@ -608,7 +634,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
     name = args.workload
 
     if world > 1:
@@ -616,7 +642,7 @@ def main():
                         world, rank, local_rank)
         return
 
-    r = measure_workload(name, W, K, local_rank, want_e2e=not args.no_e2e)
+    r = measure_workload(name, W, K, local_rank, want_e2e=not args.no_e2e, dump_dir=args.dump_outputs)
     others = {}
     if name == DEFAULT_WORKLOAD and not args.no_extra:
         for ename, ew, ek in EXTRA_WORKLOADS:

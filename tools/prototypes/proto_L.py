@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tools')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import numpy as np, scipy.sparse as sp
 from proto_pc import *
 for nx in (128,256,512):

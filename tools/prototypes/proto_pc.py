@@ -1,6 +1,6 @@
 """Prototype (scipy) of the block preconditioner to pick the algorithm before
 writing CUDA.  Not product code."""
-import sys, time; sys.path.insert(0,'/root/repo')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import numpy as np, scipy.sparse as sp, scipy.sparse.linalg as spla
 from cfd_hemodynamic_b200.fem import mesh as M, quadrature as Q
 from oracle import ns_oracle as O

@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tools')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import numpy as np, scipy.sparse as sp, scipy.sparse.linalg as spla
 from proto_pc import *
 nx=int(sys.argv[1]); mu=float(sys.argv[2]); dt=float(sys.argv[3]) if len(sys.argv)>3 else 0.01

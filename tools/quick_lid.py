@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0,'/root/repo')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from cfd_hemodynamic_b200.src.scenarios.lid_driven2D import LidDriven2DSimulation
 nx=int(sys.argv[1]); mu=float(sys.argv[2]); steps=int(sys.argv[3])
