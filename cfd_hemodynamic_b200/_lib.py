@@ -117,6 +117,7 @@ SYMBOLS = {
     "hemo_comm_allreduce": (_I, [_VP, _VP, _I]),
     "hemo_global_dot": (_I, [_VP, _VP, _VP, C.POINTER(_D)]),
     "hemo_set_poll_interval": (_I, [_VP, _I]),
+    "hemo_krylov_graph_info": (_I, [_VP, C.POINTER(_L), C.POINTER(_L)]),
 }
 
 _lib = None
@@ -462,6 +463,12 @@ class Hemo:
 
     def pc_apply(self, vals, r, z):
         self._check(self.lib.hemo_pc_apply(self._ctx, _ptr(vals), _ptr(r), _ptr(z)), "hemo_pc_apply")
+
+    def krylov_graph_info(self):
+        """(kernel nodes, programmatic-dependent-launch edges) of the last captured FGMRES iteration graph."""
+        nodes, edges = C.c_int64(), C.c_int64()
+        self._check(self.lib.hemo_krylov_graph_info(self._ctx, C.byref(nodes), C.byref(edges)), "hemo_krylov_graph_info")
+        return nodes.value, edges.value
 
     # ---- multi-GPU: NCCL inside the library ---------------------------------------
     @staticmethod

@@ -281,16 +281,22 @@ __global__ void k_max_final(int m, const double* __restrict__ partial, double* _
 
 __global__ void k_axpy_areal(int64_t n, double a, const areal* __restrict__ x, areal* __restrict__ y) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i < n) y[i] = (areal)fma(a, (double)x[i], (double)y[i]);
 }
 
 __global__ void k_to_areal(int64_t n, const double* __restrict__ x, areal* __restrict__ y) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i < n) y[i] = (areal)x[i];
 }
 
 __global__ void k_from_areal(int64_t n, const areal* __restrict__ x, double* __restrict__ y) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i < n) y[i] = (double)x[i];
 }
 
@@ -303,6 +309,8 @@ __global__ void k_cheb_start_zero(int64_t N, const areal* __restrict__ dinv, con
                                   double inv_theta, areal* __restrict__ r, areal* __restrict__ d,
                                   areal* __restrict__ x) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= N) return;
     const double rv = dinv[i] * b[i];
     r[i] = rv;
@@ -311,39 +319,55 @@ __global__ void k_cheb_start_zero(int64_t N, const areal* __restrict__ dinv, con
     x[i] = dv;
 }
 
-// (A x)_i for block row i, computed by the 4 lanes of a row group; every lane
-// of the group returns the full sum.
+// Column indices and blocks of the three strided entries a lane of a 4-lane row group handles per trip (entries beyond
+// the row end: column of the first, zero block).  The operator is constant during a solve: the first trip's chunk is
+// loaded before hemo_pdl_wait, so only the vector gathers wait for the predecessor.
 template <int BS>
-__device__ __forceinline__ void row_product(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                                            const areal* __restrict__ val, const areal* __restrict__ x,
-                                            int i, bool ok, int lane, double acc[BS]) {
-#pragma unroll
-    for (int k = 0; k < BS; ++k) acc[k] = 0.0;
-    const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
-    // The dependent chain col -> x is what bounds this kernel (rows are short): issue the
-    // column loads of three strided entries first, then the value / vector loads.
-    for (int t = r0 + lane; t < r1; t += 12) {
+struct CsrChunk {
+    int j0, j1, j2;
+    areal2 a0, a1, a2, b0, b1, b2;   // BS == 2: the two rows of each 2x2 block
+    areal v0, v1, v2;                // BS == 1
+    __device__ __forceinline__ void load(const int32_t* __restrict__ col, const areal* __restrict__ val, int t, int r1) {
         const int t1 = t + 4, t2 = t + 8;
         const bool p1 = t1 < r1, p2 = t2 < r1;
-        const int j0 = col[t];
-        const int j1 = p1 ? col[t1] : j0;
-        const int j2 = p2 ? col[t2] : j0;
+        j0 = col[t];
+        j1 = p1 ? col[t1] : j0;
+        j2 = p2 ? col[t2] : j0;
         if (BS == 1) {
-            const double v0 = (double)val[t], x0 = (double)x[j0];
-            const double v1 = p1 ? (double)val[t1] : 0.0, x1 = (double)x[j1];
-            const double v2 = p2 ? (double)val[t2] : 0.0, x2 = (double)x[j2];
-            acc[0] = fma(v0, x0, acc[0]);
-            acc[0] = fma(v1, x1, acc[0]);
-            acc[0] = fma(v2, x2, acc[0]);
+            v0 = val[t];
+            v1 = p1 ? val[t1] : (areal)0;
+            v2 = p2 ? val[t2] : (areal)0;
         } else {
             const areal2* v2p = reinterpret_cast<const areal2*>(val);
-            const areal2* x2p = reinterpret_cast<const areal2*>(x);
-            const areal2 a0 = v2p[2 * (int64_t)t], b0 = v2p[2 * (int64_t)t + 1], xa = x2p[j0];
-            areal2 a1, b1, a2, b2;
+            a0 = v2p[2 * (int64_t)t]; b0 = v2p[2 * (int64_t)t + 1];
             a1.x = a1.y = b1.x = b1.y = a2.x = a2.y = b2.x = b2.y = 0;
             if (p1) { a1 = v2p[2 * (int64_t)t1]; b1 = v2p[2 * (int64_t)t1 + 1]; }
             if (p2) { a2 = v2p[2 * (int64_t)t2]; b2 = v2p[2 * (int64_t)t2 + 1]; }
-            const areal2 xb = x2p[j1], xc = x2p[j2];
+        }
+    }
+};
+
+// (A x)_i for block row i, computed by the 4 lanes of a row group; every lane
+// of the group returns the full sum.  `ch` holds the lane's first chunk (when the row has one).
+template <int BS>
+__device__ __forceinline__ void row_product(const int32_t* __restrict__ col, const areal* __restrict__ val,
+                                            const areal* __restrict__ x, int r0, int r1, int lane, CsrChunk<BS>& ch,
+                                            double acc[BS]) {
+#pragma unroll
+    for (int k = 0; k < BS; ++k) acc[k] = 0.0;
+    // The dependent chain col -> x is what bounds this kernel (rows are short): the column
+    // loads of three strided entries are issued first, then the value / vector loads.
+    for (int t = r0 + lane; t < r1; t += 12) {
+        if (t != r0 + lane) ch.load(col, val, t, r1);
+        if (BS == 1) {
+            const double x0 = (double)x[ch.j0], x1 = (double)x[ch.j1], x2 = (double)x[ch.j2];
+            acc[0] = fma((double)ch.v0, x0, acc[0]);
+            acc[0] = fma((double)ch.v1, x1, acc[0]);
+            acc[0] = fma((double)ch.v2, x2, acc[0]);
+        } else {
+            const areal2* x2p = reinterpret_cast<const areal2*>(x);
+            const areal2 xa = x2p[ch.j0], xb = x2p[ch.j1], xc = x2p[ch.j2];
+            const areal2 a0 = ch.a0, a1 = ch.a1, a2 = ch.a2, b0 = ch.b0, b1 = ch.b1, b2 = ch.b2;
             acc[0] += (double)a0.x * xa.x + (double)a0.y * xa.y + (double)a1.x * xb.x + (double)a1.y * xb.y +
                       (double)a2.x * xc.x + (double)a2.y * xc.y;
             acc[BS - 1] += (double)b0.x * xa.x + (double)b0.y * xa.y + (double)b1.x * xb.x + (double)b1.y * xb.y +
@@ -368,8 +392,13 @@ k_cheb_start(int n, const int32_t* __restrict__ rowptr, const int32_t* __restric
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
     const int i = gt >> 2, lane = gt & 3;
     const bool ok = i < n;
+    const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
+    CsrChunk<BS> ch;
+    if (r0 + lane < r1) ch.load(col, val, r0 + lane, r1);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc[BS];
-    row_product<BS>(rowptr, col, val, xin, i, ok, lane, acc);
+    row_product<BS>(col, val, xin, r0, r1, lane, ch, acc);
     if (ok && lane < BS) {
         const int64_t q = (int64_t)i * BS + lane;
         const double rv = dinv[q] * (b[q] - (lane == 0 ? acc[0] : acc[BS - 1]));
@@ -392,29 +421,50 @@ k_presmooth_residual(int n, const int32_t* __restrict__ rowptr, const int32_t* _
     const int i = gt >> 2, lane = gt & 3;
     const bool ok = i < n;
     const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
+    // columns, blocks and inverse diagonals of two strided entries per trip; the first trip's (constant during the solve)
+    // are loaded before the wait, only the right-hand side gathers wait for the predecessor
+    int j0 = 0, j1 = 0;
+    areal2 a0, b0, a1, b1;    // BS == 2
+    areal v0 = 0, v1 = 0;     // BS == 1
+    areal d[2 * BS];
+    auto fetch = [&](int t) {
+        const int t1 = t + 4;
+        const bool p1 = t1 < r1;
+        j0 = col[t];
+        j1 = p1 ? col[t1] : j0;
+        if (BS == 1) {
+            v0 = val[t];
+            v1 = p1 ? val[t1] : (areal)0;
+        } else {
+            const areal2* v2p = reinterpret_cast<const areal2*>(val);
+            a0 = v2p[2 * (int64_t)t]; b0 = v2p[2 * (int64_t)t + 1];
+            a1.x = a1.y = b1.x = b1.y = 0;
+            if (p1) { a1 = v2p[2 * (int64_t)t1]; b1 = v2p[2 * (int64_t)t1 + 1]; }
+        }
+#pragma unroll
+        for (int k = 0; k < BS; ++k) {
+            d[k] = dinv[(int64_t)j0 * BS + k];
+            d[BS + k] = dinv[(int64_t)j1 * BS + k];
+        }
+    };
+    if (r0 + lane < r1) fetch(r0 + lane);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc[BS];
 #pragma unroll
     for (int k = 0; k < BS; ++k) acc[k] = 0.0;
     for (int t = r0 + lane; t < r1; t += 8) {
-        const int t1 = t + 4;
-        const bool p1 = t1 < r1;
-        const int j0 = col[t];
-        const int j1 = p1 ? col[t1] : j0;
+        if (t != r0 + lane) fetch(t);
         if (BS == 1) {
-            const double x0 = (double)dinv[j0] * (double)b[j0] * inv_theta;
-            const double x1 = (double)dinv[j1] * (double)b[j1] * inv_theta;
-            acc[0] = fma((double)val[t], x0, acc[0]);
-            acc[0] = fma(p1 ? (double)val[t1] : 0.0, x1, acc[0]);
+            const double x0 = (double)d[0] * (double)b[j0] * inv_theta;
+            const double x1 = (double)d[BS] * (double)b[j1] * inv_theta;
+            acc[0] = fma((double)v0, x0, acc[0]);
+            acc[0] = fma((double)v1, x1, acc[0]);
         } else {
-            const areal2* v2p = reinterpret_cast<const areal2*>(val);
-            const areal2 a0 = v2p[2 * (int64_t)t], b0 = v2p[2 * (int64_t)t + 1];
-            areal2 a1, b1;
-            a1.x = a1.y = b1.x = b1.y = 0;
-            if (p1) { a1 = v2p[2 * (int64_t)t1]; b1 = v2p[2 * (int64_t)t1 + 1]; }
-            const double xa0 = (double)dinv[2 * (int64_t)j0] * (double)b[2 * (int64_t)j0] * inv_theta;
-            const double xa1 = (double)dinv[2 * (int64_t)j0 + 1] * (double)b[2 * (int64_t)j0 + 1] * inv_theta;
-            const double xb0 = (double)dinv[2 * (int64_t)j1] * (double)b[2 * (int64_t)j1] * inv_theta;
-            const double xb1 = (double)dinv[2 * (int64_t)j1 + 1] * (double)b[2 * (int64_t)j1 + 1] * inv_theta;
+            const double xa0 = (double)d[0] * (double)b[2 * (int64_t)j0] * inv_theta;
+            const double xa1 = (double)d[1] * (double)b[2 * (int64_t)j0 + 1] * inv_theta;
+            const double xb0 = (double)d[BS] * (double)b[2 * (int64_t)j1] * inv_theta;
+            const double xb1 = (double)d[BS + 1] * (double)b[2 * (int64_t)j1 + 1] * inv_theta;
             acc[0] += (double)a0.x * xa0 + (double)a0.y * xa1 + (double)a1.x * xb0 + (double)a1.y * xb1;
             acc[BS - 1] += (double)b0.x * xa0 + (double)b0.y * xa1 + (double)b1.x * xb0 + (double)b1.y * xb1;
         }
@@ -443,8 +493,13 @@ k_cheb_step(int n, const int32_t* __restrict__ rowptr, const int32_t* __restrict
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
     const int i = gt >> 2, lane = gt & 3;
     const bool ok = i < n;
+    const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
+    CsrChunk<BS> ch;
+    if (r0 + lane < r1) ch.load(col, val, r0 + lane, r1);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc[BS];
-    row_product<BS>(rowptr, col, val, dold, i, ok, lane, acc);
+    row_product<BS>(col, val, dold, r0, r1, lane, ch, acc);
     if (ok && lane < BS) {
         const int64_t q = (int64_t)i * BS + lane;
         const double rv = r[q] - dinv[q] * (lane == 0 ? acc[0] : acc[BS - 1]);
@@ -538,48 +593,70 @@ struct JacobiLoad {
     }
 };
 
-template <int BS, typename XF>
-__device__ __forceinline__ void sell_row_product(const int32_t* __restrict__ sptr, const int32_t* __restrict__ scol,
-                                                 const areal* __restrict__ sval, int i, const XF xf, double acc[BS]) {
+// Row i of a sliced-ELL operator, consumed four trips at a time.  begin() loads the slice bounds and, with GROUP, the
+// column indices and blocks of the first four trips: the operator is constant during a solve, so a kernel issues them
+// before hemo_pdl_wait and only the vector gathers of product() wait for the predecessor.  (The pre-smoothing kernels
+// gather two vectors per entry and load nothing before the wait: holding the first group across it costs them
+// occupancy.)
+template <int BS>
+struct SellRow {
     typedef typename std::conditional<BS == 1, areal, areal4>::type blk;
-#pragma unroll
-    for (int k = 0; k < BS; ++k) acc[k] = 0.0;
-    const int s = i >> 5, lane = i & 31;
-    const int base = sptr[s];
-    const int W = (sptr[s + 1] - base) >> 5;         // uniform over the warp
-    const int32_t* __restrict__ c = scol + base + lane;
-    const blk* __restrict__ v = reinterpret_cast<const blk*>(sval) + base + lane;
-    for (int k = 0; k < W; k += 4) {
-        // trips beyond the row end repeat the last one with a zero weight
+    const int32_t* __restrict__ c;
+    const blk* __restrict__ v;
+    int W;
+    bool group;       // first group loaded by begin()
+    int j[4];
+    blk a[4];
+    template <bool GROUP>
+    __device__ __forceinline__ void begin(const int32_t* __restrict__ sptr, const int32_t* __restrict__ scol,
+                                          const areal* __restrict__ sval, int i) {
+        const int s = i >> 5, lane = i & 31;
+        const int base = sptr[s];
+        W = (sptr[s + 1] - base) >> 5;         // uniform over the warp
+        c = scol + base + lane;
+        v = reinterpret_cast<const blk*>(sval) + base + lane;
+        group = GROUP;
+        if (GROUP && W > 0) fetch(0);
+    }
+    // trips beyond the row end repeat the last one (product gives them a zero weight)
+    __device__ __forceinline__ void fetch(int k) {
         int kk[4];
-        bool ok[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) { ok[u] = k + u < W; kk[u] = 32 * (ok[u] ? k + u : W - 1); }
-        int j[4];
-        blk a[4];
-        typename XF::raw xr[4];
+        for (int u = 0; u < 4; ++u) kk[u] = 32 * (k + u < W ? k + u : W - 1);
 #pragma unroll
         for (int u = 0; u < 4; ++u) j[u] = ldg_nc(c + kk[u]);
 #pragma unroll
         for (int u = 0; u < 4; ++u) a[u] = ldg_nc(v + kk[u]);
-        __syncwarp();                    // scheduling fence: the eight loads above are in flight before the first use
+    }
+    template <typename XF>
+    __device__ __forceinline__ void product(const XF xf, double acc[BS]) {
 #pragma unroll
-        for (int u = 0; u < 4; ++u) xr[u] = xf.load(j[u]);
-        __syncwarp();
+        for (int k = 0; k < BS; ++k) acc[k] = 0.0;
+        for (int k = 0; k < W; k += 4) {
+            bool ok[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            double xv[BS];
-            xf.value(xr[u], xv);
-            if constexpr (BS == 1) {
-                acc[0] = fma(ok[u] ? (double)a[u] : 0.0, xv[0], acc[0]);
-            } else {
-                const double m = ok[u] ? 1.0 : 0.0;
-                acc[0] += m * ((double)a[u].x * xv[0] + (double)a[u].y * xv[1]);
-                acc[1] += m * ((double)a[u].z * xv[0] + (double)a[u].w * xv[1]);
+            for (int u = 0; u < 4; ++u) ok[u] = k + u < W;
+            if (k > 0 || !group) fetch(k);
+            typename XF::raw xr[4];
+            __syncwarp();                    // scheduling fence: the eight loads above are in flight before the first use
+#pragma unroll
+            for (int u = 0; u < 4; ++u) xr[u] = xf.load(j[u]);
+            __syncwarp();
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                double xv[BS];
+                xf.value(xr[u], xv);
+                if constexpr (BS == 1) {
+                    acc[0] = fma(ok[u] ? (double)a[u] : 0.0, xv[0], acc[0]);
+                } else {
+                    const double m = ok[u] ? 1.0 : 0.0;
+                    acc[0] += m * ((double)a[u].x * xv[0] + (double)a[u].y * xv[1]);
+                    acc[1] += m * ((double)a[u].z * xv[0] + (double)a[u].w * xv[1]);
+                }
             }
         }
     }
-}
+};
 
 template <int BS>
 __global__ void __launch_bounds__(256)
@@ -587,9 +664,13 @@ k_sell_cheb_start(int n, const int32_t* __restrict__ sptr, const int32_t* __rest
                   const areal* __restrict__ dinv, const areal* __restrict__ b, double inv_theta,
                   const areal* __restrict__ xin, areal* __restrict__ r, areal* __restrict__ d) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    SellRow<BS> row;
+    if (i < n) row.template begin<true>(sptr, scol, sval, i);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= n) return;
     double acc[BS];
-    sell_row_product<BS>(sptr, scol, sval, i, VecLoad<BS>{xin}, acc);
+    row.product(VecLoad<BS>{xin}, acc);
 #pragma unroll
     for (int k = 0; k < BS; ++k) {
         const int64_t q = (int64_t)i * BS + k;
@@ -605,9 +686,13 @@ k_sell_presmooth_residual(int n, const int32_t* __restrict__ sptr, const int32_t
                           const areal* __restrict__ sval, const areal* __restrict__ dinv, const TB* __restrict__ b,
                           double inv_theta, areal* __restrict__ x, areal* __restrict__ r, areal* __restrict__ bcopy) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= n) return;
+    SellRow<BS> row;
+    row.template begin<false>(sptr, scol, sval, i);
     double acc[BS];
-    sell_row_product<BS>(sptr, scol, sval, i, JacobiLoad<BS, TB>{dinv, b, inv_theta}, acc);
+    row.product(JacobiLoad<BS, TB>{dinv, b, inv_theta}, acc);
 #pragma unroll
     for (int k = 0; k < BS; ++k) {
         const int64_t q = (int64_t)i * BS + k;
@@ -625,9 +710,13 @@ k_sell_cheb_step(int n, const int32_t* __restrict__ sptr, const int32_t* __restr
                  areal* __restrict__ dnew, areal* __restrict__ r, areal* __restrict__ x, int add_old,
                  double* __restrict__ x64) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    SellRow<BS> row;
+    if (i < n) row.template begin<true>(sptr, scol, sval, i);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= n) return;
     double acc[BS];
-    sell_row_product<BS>(sptr, scol, sval, i, VecLoad<BS>{dold}, acc);
+    row.product(VecLoad<BS>{dold}, acc);
 #pragma unroll
     for (int k = 0; k < BS; ++k) {
         const int64_t q = (int64_t)i * BS + k;
@@ -648,9 +737,13 @@ __global__ void __launch_bounds__(256)
 k_sell_residual(int n, const int32_t* __restrict__ sptr, const int32_t* __restrict__ scol, const areal* __restrict__ sval,
                 const areal* __restrict__ x, const areal* __restrict__ b, areal* __restrict__ y) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    SellRow<BS> row;
+    if (i < n) row.template begin<true>(sptr, scol, sval, i);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= n) return;
     double acc[BS];
-    sell_row_product<BS>(sptr, scol, sval, i, VecLoad<BS>{x}, acc);
+    row.product(VecLoad<BS>{x}, acc);
 #pragma unroll
     for (int k = 0; k < BS; ++k) {
         const int64_t q = (int64_t)i * BS + k;
@@ -693,14 +786,19 @@ __global__ void __launch_bounds__(256)
 k_prolong_add_row(int nrows, const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                   const double* __restrict__ w, const areal* __restrict__ x, areal* __restrict__ y) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nrows) return;
-    const int r0 = rowptr[i], r1 = rowptr[i + 1];
+    const bool ok = i < nrows;
+    const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
+    int j = 0;
+    double wt = 0.0;
+    if (r0 < r1) { j = col[r0]; wt = w[r0]; }       // first entry (constant) before the wait
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
+    if (!ok) return;
     double acc[BS];
 #pragma unroll
     for (int k = 0; k < BS; ++k) acc[k] = 0.0;
     for (int t = r0; t < r1; ++t) {
-        const int j = col[t];
-        const double wt = w[t];
+        if (t != r0) { j = col[t]; wt = w[t]; }
 #pragma unroll
         for (int k = 0; k < BS; ++k) acc[k] = fma(wt, (double)x[(int64_t)j * BS + k], acc[k]);
     }
@@ -721,16 +819,25 @@ k_transfer(int nrows, const int32_t* __restrict__ rowptr, const int32_t* __restr
     const int I = gt >> 2, lane = gt & 3;
     const bool ok = I < nrows;
     const int r0 = ok ? rowptr[I] : 0, r1 = ok ? rowptr[I + 1] : 0;
+    // the first trip's columns and weights (constant) before the wait
+    int j0 = 0, j1 = 0, j2 = 0;
+    double w0 = 0.0, w1 = 0.0, w2 = 0.0;
+    auto fetch = [&](int t) {
+        const int t1 = t + 4, t2 = t + 8;
+        const bool p1 = t1 < r1, p2 = t2 < r1;
+        j0 = col[t];
+        j1 = p1 ? col[t1] : j0;
+        j2 = p2 ? col[t2] : j0;
+        w0 = w[t]; w1 = p1 ? w[t1] : 0.0; w2 = p2 ? w[t2] : 0.0;
+    };
+    if (r0 + lane < r1) fetch(r0 + lane);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc[BS];
 #pragma unroll
     for (int k = 0; k < BS; ++k) acc[k] = 0.0;
     for (int t = r0 + lane; t < r1; t += 12) {
-        const int t1 = t + 4, t2 = t + 8;
-        const bool p1 = t1 < r1, p2 = t2 < r1;
-        const int j0 = col[t];
-        const int j1 = p1 ? col[t1] : j0;
-        const int j2 = p2 ? col[t2] : j0;
-        const double w0 = w[t], w1 = p1 ? w[t1] : 0.0, w2 = p2 ? w[t2] : 0.0;
+        if (t != r0 + lane) fetch(t);
 #pragma unroll
         for (int k = 0; k < BS; ++k) {
             const double x0 = (double)x[(int64_t)j0 * BS + k], x1 = (double)x[(int64_t)j1 * BS + k],
@@ -972,6 +1079,8 @@ template <int BS>
 __global__ void __launch_bounds__(1024)
 k_coarse_vcycle(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
                 int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     CtaScope sc;
     coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, degree_pre, degree, ratio, dense_inv, dense_n);
 }
@@ -1058,6 +1167,8 @@ __global__ void __launch_bounds__(256)
 k_dense_gemv(int N, const double* __restrict__ inv, const areal* __restrict__ b, areal* __restrict__ y) {
     const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc = 0.0;
     if (row < N)
         for (int c = lane; c < N; c += 32) acc += inv[(int64_t)row * N + c] * b[c];
@@ -1427,15 +1538,14 @@ static int smooth_t(hemo_ctx* ctx, const HemoAmgOp& A, const areal* b, areal* x,
     areal* d0 = A.d;
     areal* d1 = A.d + N;
     if (x_is_zero) {
-        k_cheb_start_zero<BS><<<hemo_grid(N, 256), 256, 0, st>>>(N, A.dinv, b, 1.0 / theta, A.r, d0, x);
+        HEMO_LAUNCH(ctx, k_cheb_start_zero<BS>, hemo_grid(N, 256), 256, 0, st, N, A.dinv, b, 1.0 / theta, A.r, d0, x);
     } else if (A.sell_ptr) {
-        k_sell_cheb_start<BS><<<hemo_grid(A.n, 256), 256, 0, st>>>(A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, b, 1.0 / theta,
-                                                                    x, A.r, d0);
+        HEMO_LAUNCH(ctx, k_sell_cheb_start<BS>, hemo_grid(A.n, 256), 256, 0, st, A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, b,
+                    1.0 / theta, x, A.r, d0);
     } else {
-        k_cheb_start<BS><<<hemo_grid((int64_t)A.n * 4, 256), 256, 0, st>>>(A.n, A.rowptr, A.col, A.val, A.dinv, b, 1.0 / theta, x,
-                                                              A.r, d0);
+        HEMO_LAUNCH(ctx, k_cheb_start<BS>, hemo_grid((int64_t)A.n * 4, 256), 256, 0, st, A.n, A.rowptr, A.col, A.val, A.dinv, b,
+                    1.0 / theta, x, A.r, d0);
     }
-    HEMO_LAUNCH_CHECK(ctx);
     bool pending = !x_is_zero;   // x += d0 still to be applied
     for (int k = 1; k < degree; ++k) {
         const double rho_new = 1.0 / (2.0 * sigma - rho);
@@ -1444,22 +1554,18 @@ static int smooth_t(hemo_ctx* ctx, const HemoAmgOp& A, const areal* b, areal* x,
         if (fine) HEMO_PROF_BEGIN(ctx, BS == 2 ? HEMO_PROF_CHEB_U0 : HEMO_PROF_CHEB_P0);
         const bool last = (k == degree - 1);
         if (A.sell_ptr)
-            k_sell_cheb_step<BS><<<hemo_grid(A.n, 256), 256, 0, st>>>(A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, c1, c2, d0, d1,
-                                                                       A.r, x, pending ? 1 : 0, last ? x64 : nullptr);
+            HEMO_LAUNCH(ctx, k_sell_cheb_step<BS>, hemo_grid(A.n, 256), 256, 0, st, A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, c1,
+                        c2, d0, d1, A.r, x, pending ? 1 : 0, last ? x64 : nullptr);
         else
-            k_cheb_step<BS><<<hemo_grid((int64_t)A.n * 4, 256), 256, 0, st>>>(A.n, A.rowptr, A.col, A.val, A.dinv, c1, c2, d0, d1, A.r, x,
-                                                                 pending ? 1 : 0, last ? x64 : nullptr);
+            HEMO_LAUNCH(ctx, k_cheb_step<BS>, hemo_grid((int64_t)A.n * 4, 256), 256, 0, st, A.n, A.rowptr, A.col, A.val, A.dinv, c1, c2,
+                        d0, d1, A.r, x, pending ? 1 : 0, last ? x64 : nullptr);
         if (last && x64 && wrote64) *wrote64 = true;
-        HEMO_LAUNCH_CHECK(ctx);
         if (fine) HEMO_PROF_END(ctx, BS == 2 ? HEMO_PROF_CHEB_U0 : HEMO_PROF_CHEB_P0);
         pending = false;
         areal* t = d0; d0 = d1; d1 = t;
         rho = rho_new;
     }
-    if (pending) {
-        k_axpy_areal<<<hemo_grid(N, 256), 256, 0, st>>>(N, 1.0, d0, x);
-        HEMO_LAUNCH_CHECK(ctx);
-    }
+    if (pending) HEMO_LAUNCH(ctx, k_axpy_areal, hemo_grid(N, 256), 256, 0, st, N, 1.0, d0, x);
     return 0;
 }
 
@@ -1506,16 +1612,14 @@ static int vcycle_t(hemo_ctx* ctx, HemoAmg* amg, int l, const areal* b, areal* x
     }
     if (l == amg->fuse_level) {
         // every remaining level fits one CTA
-        k_coarse_vcycle<BS><<<1, 1024, 0, st>>>(amg->fuse_desc + (l - amg->fuse_base), amg->nlev - l, b, x, degree_pre, degree, ratio,
-                                                amg->dense_inv, amg->dense_n);
-        HEMO_LAUNCH_CHECK(ctx);
+        HEMO_LAUNCH(ctx, k_coarse_vcycle<BS>, 1, 1024, 0, st, amg->fuse_desc + (l - amg->fuse_base), amg->nlev - l, b, x, degree_pre,
+                    degree, ratio, amg->dense_inv, amg->dense_n);
         return 0;
     }
     if (l == amg->nlev - 1) {
         const int N = amg->dense_n;
         // exact solve: any previous iterate is simply replaced
-        k_dense_gemv<<<hemo_grid((int64_t)N * 32, 256), 256, 0, st>>>(N, amg->dense_inv, b, x);
-        HEMO_LAUNCH_CHECK(ctx);
+        HEMO_LAUNCH(ctx, k_dense_gemv, hemo_grid((int64_t)N * 32, 256), 256, 0, st, N, amg->dense_inv, b, x);
         return 0;
     }
     int rc;
@@ -1524,39 +1628,38 @@ static int vcycle_t(hemo_ctx* ctx, HemoAmg* amg, int l, const areal* b, areal* x
         const double lmax = A.lmax, lmin = lmax / ratio;
         const double inv_theta = 1.0 / (0.5 * (lmax + lmin));
         const int g = hemo_grid((int64_t)A.n * 4, 256);
+        areal* const no_copy = nullptr;
         if (A.sell_ptr) {
             const int gs = hemo_grid(A.n, 256);
-            if (b64) k_sell_presmooth_residual<BS, double><<<gs, 256, 0, st>>>(A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, b64,
-                                                                                inv_theta, x, A.r, const_cast<areal*>(b));
-            else k_sell_presmooth_residual<BS, areal><<<gs, 256, 0, st>>>(A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv, b,
-                                                                          inv_theta, x, A.r, nullptr);
-        } else if (b64) k_presmooth_residual<BS, double><<<g, 256, 0, st>>>(A.n, A.rowptr, A.col, A.val, A.dinv, b64, inv_theta, x, A.r,
-                                                                      const_cast<areal*>(b));
-        else k_presmooth_residual<BS, areal><<<g, 256, 0, st>>>(A.n, A.rowptr, A.col, A.val, A.dinv, b, inv_theta, x, A.r, nullptr);
-        HEMO_LAUNCH_CHECK(ctx);
+            if (b64) HEMO_LAUNCH(ctx, (k_sell_presmooth_residual<BS, double>), gs, 256, 0, st, A.n, A.sell_ptr, A.sell_col, A.sell_val,
+                                 A.dinv, b64, inv_theta, x, A.r, const_cast<areal*>(b));
+            else HEMO_LAUNCH(ctx, (k_sell_presmooth_residual<BS, areal>), gs, 256, 0, st, A.n, A.sell_ptr, A.sell_col, A.sell_val, A.dinv,
+                             b, inv_theta, x, A.r, no_copy);
+        } else if (b64) HEMO_LAUNCH(ctx, (k_presmooth_residual<BS, double>), g, 256, 0, st, A.n, A.rowptr, A.col, A.val, A.dinv, b64,
+                                    inv_theta, x, A.r, const_cast<areal*>(b));
+        else HEMO_LAUNCH(ctx, (k_presmooth_residual<BS, areal>), g, 256, 0, st, A.n, A.rowptr, A.col, A.val, A.dinv, b, inv_theta, x,
+                         A.r, no_copy);
     } else {
         if (b64) {          // the fused kernel is not used: convert the right-hand side first
             const int64_t N = (int64_t)A.n * BS;
-            k_to_areal<<<hemo_grid(N, 256), 256, 0, st>>>(N, b64, const_cast<areal*>(b));
-            HEMO_LAUNCH_CHECK(ctx);
+            HEMO_LAUNCH(ctx, k_to_areal, hemo_grid(N, 256), 256, 0, st, N, b64, const_cast<areal*>(b));
         }
         if ((rc = smooth_t<BS>(ctx, A, b, x, x_is_zero, degree_pre, ratio))) return rc;
         // residual and restriction
         if (A.sell_ptr) {
-            k_sell_residual<BS><<<hemo_grid(A.n, 256), 256, 0, st>>>(A.n, A.sell_ptr, A.sell_col, A.sell_val, x, b, A.r);
-            HEMO_LAUNCH_CHECK(ctx);
+            HEMO_LAUNCH(ctx, k_sell_residual<BS>, hemo_grid(A.n, 256), 256, 0, st, A.n, A.sell_ptr, A.sell_col, A.sell_val, x, b, A.r);
         } else if ((rc = hemo_bsr_spmv_ex(ctx, BS, A.n, A.rowptr, A.col, A.val, x, -1.0, b, A.r))) return rc;
     }
     const HemoAmgLevel& L = amg->lev[l];
     HemoAmgOp& C = amg->op[l + 1];
-    k_transfer<BS, false><<<hemo_grid((int64_t)C.n * 4, 256), 256, 0, st>>>(C.n, L.r_rowptr, L.r_col, L.r_val, A.r, C.b);
-    HEMO_LAUNCH_CHECK(ctx);
+    HEMO_LAUNCH(ctx, (k_transfer<BS, false>), hemo_grid((int64_t)C.n * 4, 256), 256, 0, st, C.n, L.r_rowptr, L.r_col, L.r_val, A.r,
+                C.b);
     if ((rc = vcycle_t<BS>(ctx, amg, l + 1, C.b, C.x, true))) return rc;
     if (L.nnz_p <= 6 * (int64_t)A.n && A.n >= 32768)
-        k_prolong_add_row<BS><<<hemo_grid(A.n, 256), 256, 0, st>>>(A.n, L.p_rowptr, L.p_col, L.p_val, C.x, x);
+        HEMO_LAUNCH(ctx, k_prolong_add_row<BS>, hemo_grid(A.n, 256), 256, 0, st, A.n, L.p_rowptr, L.p_col, L.p_val, C.x, x);
     else
-        k_transfer<BS, true><<<hemo_grid((int64_t)A.n * 4, 256), 256, 0, st>>>(A.n, L.p_rowptr, L.p_col, L.p_val, C.x, x);
-    HEMO_LAUNCH_CHECK(ctx);
+        HEMO_LAUNCH(ctx, (k_transfer<BS, true>), hemo_grid((int64_t)A.n * 4, 256), 256, 0, st, A.n, L.p_rowptr, L.p_col, L.p_val, C.x,
+                    x);
     if ((rc = smooth_t<BS>(ctx, A, b, x, false, degree, ratio, x64, wrote64))) return rc;
     return 0;
 }
@@ -1572,10 +1675,7 @@ int hemo_amg_vcycle(hemo_ctx* ctx, HemoAmg* amg, const double* b, double* x, int
     // the top level runs per-level kernels (not inside a fused kernel, not the dense coarsest solve): its first kernel
     // reads the fp64 right-hand side and its last one writes the fp64 result — no conversion kernels
     const bool per_level_top = amg->nlev > 1 && amg->fuse_level != 0 && !(amg->fuse_level_grid == 0 && amg->grid_blocks > 0);
-    if (!per_level_top) {
-        k_to_areal<<<hemo_grid(N, 256), 256, 0, ctx->stream>>>(N, b, top.b);
-        HEMO_LAUNCH_CHECK(ctx);
-    }
+    if (!per_level_top) HEMO_LAUNCH(ctx, k_to_areal, hemo_grid(N, 256), 256, 0, ctx->stream, N, b, top.b);
     bool wrote64 = false;
     for (int c = 0; c < nc; ++c) {
         const double* b64 = (per_level_top && c == 0) ? b : nullptr;
@@ -1584,9 +1684,6 @@ int hemo_amg_vcycle(hemo_ctx* ctx, HemoAmg* amg, const double* b, double* x, int
         else rc = vcycle_t<1>(ctx, amg, 0, top.b, top.x, c == 0, b64, x64, &wrote64);
         if (rc) return rc;
     }
-    if (!wrote64) {
-        k_from_areal<<<hemo_grid(N, 256), 256, 0, ctx->stream>>>(N, top.x, x);
-        HEMO_LAUNCH_CHECK(ctx);
-    }
+    if (!wrote64) HEMO_LAUNCH(ctx, k_from_areal, hemo_grid(N, 256), 256, 0, ctx->stream, N, top.x, x);
     return 0;
 }

@@ -119,6 +119,8 @@ extern "C" int hemo_comm_init(hemo_ctx* ctx, const char* uid128, int rank, int n
         return 1000 + (int)r;
     }
     ctx->comm = c;
+    // the partitioned solve keeps plain launches: its chains interleave NCCL collectives with the library's kernels
+    ctx->pdl = 0;
     return 0;
 }
 

@@ -168,6 +168,8 @@ struct HemoKrylov {
     bool iter_valid = false;
     const double* iter_vals = nullptr;
     int64_t iter_nodes = 0;
+    // kernel nodes and programmatic (PDL) edges of the last captured iteration graph (hemo_krylov_graph_info)
+    int64_t iter_kernel_nodes = 0, iter_prog_edges = 0;
 };
 
 struct hemo_ctx {
@@ -180,6 +182,7 @@ struct hemo_ctx {
     cudaStream_t stream = 0;
     std::string err;
     int64_t launches = 0;
+    int pdl = 1;                     // programmatic dependent launch of the iteration kernels (HEMO_PDL=0 turns it off)
 
     // mesh (borrowed)
     int nv = 3;                     // nodes per cell: 3 = P1 triangle, 4 = Q1 quadrilateral (tensor-ordered) | P1 tetrahedron,
@@ -309,6 +312,76 @@ struct hemo_ctx {
                          cudaGetErrorString(_e) + " at " + __FILE__ + ":" + std::to_string(__LINE__); \
             return (int)_e;                                          \
         }                                                            \
+    } while (0)
+
+// Programmatic dependent launch (PDL).  A kernel launched by HEMO_LAUNCH on a context with `pdl` set may be dispatched
+// while its stream predecessor still runs.  Such a kernel follows one protocol:
+//   1. optionally, loads of operands no kernel of the solve writes (operator values, indices, transfer weights);
+//   2. hemo_pdl_wait(), unconditionally and before any early return: it blocks until the predecessor grid has completed
+//      and its writes are visible, so the grid never completes ahead of its predecessor;
+//   3. hemo_pdl_trigger(), which lets the successor's CTAs be dispatched (wait before trigger keeps at most two grids
+//      of the chain live, so step 1 only ever overlaps the immediate predecessor);
+//   4. the body.
+// Both are no-ops in a kernel launched without the attribute.
+__device__ __forceinline__ void hemo_pdl_wait() {
+#if defined(__CUDA_ARCH__) && __CUDA_ARCH__ >= 900
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+#endif
+}
+__device__ __forceinline__ void hemo_pdl_trigger() {
+#if defined(__CUDA_ARCH__) && __CUDA_ARCH__ >= 900
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+#endif
+}
+
+// Whether a launch on `st` may carry the programmatic-serialization attribute.  During stream capture the attribute
+// becomes a programmatic graph edge, which only exists between kernel nodes: after a memcpy, an event join (several
+// dependencies) or the start of the capture the launch stays plain.
+static inline bool hemo_pdl_allowed(cudaStream_t st) {
+    if (st == 0) return false;
+    cudaStreamCaptureStatus cs;
+    const cudaGraphNode_t* deps = nullptr;
+    size_t nd = 0;
+    if (cudaStreamGetCaptureInfo(st, &cs, nullptr, nullptr, &deps, &nd) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    if (cs != cudaStreamCaptureStatusActive) return true;
+    cudaGraphNodeType t;
+    return nd == 1 && cudaGraphNodeGetType(deps[0], &t) == cudaSuccess && t == cudaGraphNodeTypeKernel;
+}
+
+template <typename... P, typename... A>
+static inline cudaError_t hemo_launch_kernel(hemo_ctx* ctx, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem,
+                                             cudaStream_t st, A... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    if (ctx->pdl && hemo_pdl_allowed(st)) {
+        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
+    }
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
+    const cudaError_t last = cudaGetLastError();
+    return e != cudaSuccess ? e : last;
+}
+
+// kernel<<<grid, block, smem, st>>>(args...) followed by HEMO_LAUNCH_CHECK, for kernels that follow the PDL protocol
+// above.  A template-id with a comma goes in parentheses: HEMO_LAUNCH(ctx, (k<BS, double>), ...).
+#define HEMO_LAUNCH(ctx, kernel, grid, block, smem, st, ...)                                                        \
+    do {                                                                                                            \
+        (ctx)->launches++;                                                                                          \
+        cudaError_t _e = hemo_launch_kernel((ctx), kernel, dim3(grid), dim3(block), (size_t)(smem), (st), __VA_ARGS__); \
+        if (_e != cudaSuccess) {                                                                                    \
+            (ctx)->err = std::string("kernel launch: ") +                                                           \
+                         cudaGetErrorString(_e) + " at " + __FILE__ + ":" + std::to_string(__LINE__);              \
+            return (int)_e;                                                                                         \
+        }                                                                                                           \
     } while (0)
 
 static inline void hemo_prof_mark(hemo_ctx* ctx, int cls) {

@@ -132,6 +132,8 @@ __global__ void k_fg_begin_cycle(FgState* st, const double* __restrict__ normsq,
 __global__ void __launch_bounds__(FG_THREADS)
 k_fg_load(const FgState* __restrict__ st, int64_t n, const double* __restrict__ V, int64_t ldv,
           const double* __restrict__ scale, double* __restrict__ pc_in) {
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     const int j = st->j;
     const double s = scale[j];
@@ -145,12 +147,6 @@ __global__ void __launch_bounds__(256)
 k_fg_spmv_node(const FgState* __restrict__ st, int n, int64_t nnz_node, const int32_t* __restrict__ nrowptr,
                const int32_t* __restrict__ ncol, const double* __restrict__ vals, const double* __restrict__ z,
                double* __restrict__ V, double* __restrict__ Z, int64_t ldv) {
-    if (st->converged || st->cycle_full) return;
-    const int j = st->j;
-    const double* xu = z;
-    const double* xp = z + 2 * (int64_t)n;
-    double* w = V + (int64_t)(j + 1) * ldv;
-    double* zj = Z + (int64_t)j * ldv;
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
     const int i = gt >> 3;
     const int lane = gt & 7;
@@ -158,14 +154,32 @@ k_fg_spmv_node(const FgState* __restrict__ st, int n, int64_t nnz_node, const in
     const int r0 = ok ? nrowptr[i] : 0;
     const int deg = ok ? nrowptr[i + 1] - r0 : 0;
     const int64_t ru0 = 6 * (int64_t)r0, ru1 = ru0 + 3 * deg, rp = 6 * nnz_node + 3 * (int64_t)r0;
+    // the first trip's column index and Jacobian entries (constant during the solve) load before the wait
+    int c = 0;
+    double v[9];
+    auto fetch = [&](int t) {
+        c = ncol[r0 + t];
+        v[0] = vals[ru0 + 2 * t]; v[1] = vals[ru0 + 2 * t + 1]; v[2] = vals[ru0 + 2 * deg + t];
+        v[3] = vals[ru1 + 2 * t]; v[4] = vals[ru1 + 2 * t + 1]; v[5] = vals[ru1 + 2 * deg + t];
+        v[6] = vals[rp + 2 * t];  v[7] = vals[rp + 2 * t + 1];  v[8] = vals[rp + 2 * deg + t];
+    };
+    if (lane < deg) fetch(lane);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
+    if (st->converged || st->cycle_full) return;
+    const int j = st->j;
+    const double* xu = z;
+    const double* xp = z + 2 * (int64_t)n;
+    double* w = V + (int64_t)(j + 1) * ldv;
+    double* zj = Z + (int64_t)j * ldv;
     double a0 = 0.0, a1 = 0.0, a2 = 0.0;
     for (int t = lane; t < deg; t += 8) {
-        const int c = ncol[r0 + t];
+        if (t != lane) fetch(t);
         const double2 xv = reinterpret_cast<const double2*>(xu)[c];
         const double x2 = xp[c];
-        a0 += vals[ru0 + 2 * t] * xv.x + vals[ru0 + 2 * t + 1] * xv.y + vals[ru0 + 2 * deg + t] * x2;
-        a1 += vals[ru1 + 2 * t] * xv.x + vals[ru1 + 2 * t + 1] * xv.y + vals[ru1 + 2 * deg + t] * x2;
-        a2 += vals[rp + 2 * t] * xv.x + vals[rp + 2 * t + 1] * xv.y + vals[rp + 2 * deg + t] * x2;
+        a0 += v[0] * xv.x + v[1] * xv.y + v[2] * x2;
+        a1 += v[3] * xv.x + v[4] * xv.y + v[5] * x2;
+        a2 += v[6] * xv.x + v[7] * xv.y + v[8] * x2;
     }
 #pragma unroll
     for (int o = 4; o > 0; o >>= 1) {
@@ -185,6 +199,8 @@ k_fg_spmv_node(const FgState* __restrict__ st, int n, int64_t nnz_node, const in
 __global__ void __launch_bounds__(FG_THREADS)
 k_fg_store(const FgState* __restrict__ st, int64_t n, const double* __restrict__ z, const double* __restrict__ w,
            double* __restrict__ V, double* __restrict__ Z, int64_t ldv) {
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     const int j = st->j;
     double* wj = V + (int64_t)(j + 1) * ldv;
@@ -203,6 +219,8 @@ __global__ void __launch_bounds__(FG_THREADS)
 k_fg_mdot(const FgState* __restrict__ st, FgSeg seg, const double* __restrict__ V, int64_t ldv,
           double* __restrict__ partial /*[m+1][gridDim.x]*/, int kpad) {
     extern __shared__ double acc_sh[];       // (FG_THREADS / 32) x kpad
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     const int j = st->j, k = j + 1;
     const double* w = V + (int64_t)k * ldv;
@@ -266,6 +284,8 @@ __global__ void __launch_bounds__(128)
 k_fg_mdot_final(const FgState* __restrict__ st, int nblk, const double* __restrict__ partial,
                 const double* __restrict__ scale, double* __restrict__ hcol) {
     __shared__ double sh[32];
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     const int i = blockIdx.x;
     if (i > st->j) return;
@@ -330,6 +350,8 @@ k_fg_maxpy(FgState* st, FgSeg seg, int64_t nloc, double* __restrict__ V, int64_t
            double* __restrict__ cs, double* __restrict__ sn, double* __restrict__ g, double* __restrict__ scale) {
     __shared__ double sh[32];
     extern __shared__ double hsh[];
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     const int j = st->j, k = j + 1;
     double* w = V + (int64_t)k * ldv;
@@ -362,6 +384,8 @@ __global__ void k_fg_givens(FgState* st, int m, const double* __restrict__ hcol,
                             double* __restrict__ H, double* __restrict__ cs, double* __restrict__ sn,
                             double* __restrict__ g, double* __restrict__ scale) {
     extern __shared__ double gsh[];
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
     fg_givens(st, m, hcol, sqrt(fmax(normsq[0], 0.0)), H, cs, sn, g, scale, gsh);
 }
@@ -480,8 +504,7 @@ static int fg_iteration_body(hemo_ctx* ctx, const double* vals_dev) {
     cudaStream_t st = ctx->stream;
     const FgSeg seg = {K.seg_len0 ? K.seg_len0 : N, K.seg_off1, K.seg_len0 ? K.seg_len1 : 0};
     int rc;
-    k_fg_load<<<fg_grid(N, 4), FG_THREADS, 0, st>>>(p.st, N, ctx->kry_V, ldv, p.scale, ctx->pc_in);
-    HEMO_LAUNCH_CHECK(ctx);
+    HEMO_LAUNCH(ctx, k_fg_load, fg_grid(N, 4), FG_THREADS, 0, st, p.st, N, ctx->kry_V, ldv, p.scale, ctx->pc_in);
     if (ctx->comm && ctx->comm_ras_overlap && (rc = hemo_comm_halo(ctx, ctx->pc_in))) return rc;
     HEMO_PROF_BEGIN(ctx, HEMO_PROF_PC);
     if ((rc = hemo_pc_apply_body(ctx, vals_dev, ctx->pc_in, ctx->pc_out))) return rc;
@@ -490,12 +513,12 @@ static int fg_iteration_body(hemo_ctx* ctx, const double* vals_dev) {
     HEMO_PROF_BEGIN(ctx, HEMO_PROF_SPMV);
     if (ctx->dim == 3) {
         if ((rc = hemo_tet_spmv(ctx, vals_dev, ctx->pc_out, ctx->kry_w))) return rc;
-        k_fg_store<<<fg_grid(N, 4), FG_THREADS, 0, st>>>(p.st, N, ctx->pc_out, ctx->kry_w, ctx->kry_V, ctx->kry_Z, ldv);
+        HEMO_LAUNCH(ctx, k_fg_store, fg_grid(N, 4), FG_THREADS, 0, st, p.st, N, ctx->pc_out, ctx->kry_w, ctx->kry_V, ctx->kry_Z,
+                    ldv);
     } else {
-        k_fg_spmv_node<<<hemo_grid((int64_t)n * 8, 256), 256, 0, st>>>(p.st, n, ctx->nnz_node, ctx->nrowptr, ctx->ncol, vals_dev,
-                                                                    ctx->pc_out, ctx->kry_V, ctx->kry_Z, ldv);
+        HEMO_LAUNCH(ctx, k_fg_spmv_node, hemo_grid((int64_t)n * 8, 256), 256, 0, st, p.st, n, ctx->nnz_node, ctx->nrowptr,
+                    ctx->ncol, vals_dev, ctx->pc_out, ctx->kry_V, ctx->kry_Z, ldv);
     }
-    HEMO_LAUNCH_CHECK(ctx);
     HEMO_PROF_END(ctx, HEMO_PROF_SPMV);
     const int64_t nown = seg.len0 + seg.len1;
     HEMO_PROF_BEGIN(ctx, HEMO_PROF_MDOT);
@@ -503,26 +526,45 @@ static int fg_iteration_body(hemo_ctx* ctx, const double* vals_dev) {
         const int kpad = m + 4;
         const int gm = fg_grid(nown, FG_TILE);
         const size_t smem = sizeof(double) * (FG_THREADS / 32) * kpad;
-        if (seg.len1 > 0) k_fg_mdot<true><<<gm, FG_THREADS, smem, st>>>(p.st, seg, ctx->kry_V, ldv, K.partial, kpad);
-        else k_fg_mdot<false><<<gm, FG_THREADS, smem, st>>>(p.st, seg, ctx->kry_V, ldv, K.partial, kpad);
-        HEMO_LAUNCH_CHECK(ctx);
-        k_fg_mdot_final<<<m, 128, 0, st>>>(p.st, gm, K.partial, p.scale, p.hcol);
-        HEMO_LAUNCH_CHECK(ctx);
+        if (seg.len1 > 0) HEMO_LAUNCH(ctx, k_fg_mdot<true>, gm, FG_THREADS, smem, st, p.st, seg, ctx->kry_V, ldv, K.partial, kpad);
+        else HEMO_LAUNCH(ctx, k_fg_mdot<false>, gm, FG_THREADS, smem, st, p.st, seg, ctx->kry_V, ldv, K.partial, kpad);
+        HEMO_LAUNCH(ctx, k_fg_mdot_final, m, 128, 0, st, p.st, gm, K.partial, p.scale, p.hcol);
     }
     HEMO_PROF_END(ctx, HEMO_PROF_MDOT);
     if (ctx->comm && (rc = hemo_comm_allreduce_j(ctx, p.hcol, m + 1))) return rc;
     HEMO_PROF_BEGIN(ctx, HEMO_PROF_MAXPY);
-    k_fg_maxpy<<<fg_grid(N, 1), FG_THREADS, sizeof(double) * 3 * (m + 2), st>>>(p.st, seg, N, ctx->kry_V, ldv, p.hcol, m, K.partial,
-                                                                               p.normsq, ctx->comm ? 0 : 1, p.H, p.cs, p.sn, p.g,
-                                                                               p.scale);
-    HEMO_LAUNCH_CHECK(ctx);
+    HEMO_LAUNCH(ctx, k_fg_maxpy, fg_grid(N, 1), FG_THREADS, sizeof(double) * 3 * (m + 2), st, p.st, seg, N, ctx->kry_V, ldv,
+                p.hcol, m, K.partial, p.normsq, ctx->comm ? 0 : 1, p.H, p.cs, p.sn, p.g, p.scale);
     HEMO_PROF_END(ctx, HEMO_PROF_MAXPY);
     if (ctx->comm) {
         if ((rc = hemo_comm_allreduce_j(ctx, p.normsq, 1))) return rc;
-        k_fg_givens<<<1, 64, sizeof(double) * 3 * (m + 2), st>>>(p.st, m, p.hcol, p.normsq, p.H, p.cs, p.sn, p.g, p.scale);
-        HEMO_LAUNCH_CHECK(ctx);
+        HEMO_LAUNCH(ctx, k_fg_givens, 1, 64, sizeof(double) * 3 * (m + 2), st, p.st, m, p.hcol, p.normsq, p.H, p.cs, p.sn, p.g,
+                    p.scale);
     }
     return 0;
+}
+
+// kernel nodes and programmatic-dependency edges of a captured graph
+static void fg_graph_stats(cudaGraph_t g, int64_t* kernels, int64_t* prog) {
+    *kernels = *prog = 0;
+    size_t nn = 0, ne = 0;
+    if (cudaGraphGetNodes(g, nullptr, &nn) != cudaSuccess || cudaGraphGetEdges_v2(g, nullptr, nullptr, nullptr, &ne) != cudaSuccess) {
+        cudaGetLastError();
+        return;
+    }
+    std::vector<cudaGraphNode_t> nodes(nn), from(ne), to(ne);
+    std::vector<cudaGraphEdgeData> data(ne);
+    if (cudaGraphGetNodes(g, nodes.data(), &nn) != cudaSuccess ||
+        cudaGraphGetEdges_v2(g, from.data(), to.data(), data.data(), &ne) != cudaSuccess) {
+        cudaGetLastError();
+        return;
+    }
+    for (cudaGraphNode_t v : nodes) {
+        cudaGraphNodeType t;
+        if (cudaGraphNodeGetType(v, &t) == cudaSuccess && t == cudaGraphNodeTypeKernel) ++*kernels;
+    }
+    for (const cudaGraphEdgeData& d : data)
+        if (d.type == cudaGraphDependencyTypeProgrammatic) ++*prog;
 }
 
 // The iteration replays as one CUDA graph (captured once per preconditioner set-up: the kernel arguments do not
@@ -558,6 +600,7 @@ static int fg_iteration(hemo_ctx* ctx, const double* vals_dev) {
         ctx->use_graph = 0;
         return fg_iteration_body(ctx, vals_dev);
     }
+    fg_graph_stats(g, &K.iter_kernel_nodes, &K.iter_prog_edges);
     bool updated = false;
     if (K.iter_exec) {
         cudaGraphExecUpdateResultInfo info;
@@ -573,6 +616,14 @@ static int fg_iteration(hemo_ctx* ctx, const double* vals_dev) {
     K.iter_vals = vals_dev;
     HEMO_CHECK_CUDA(ctx, cudaGraphLaunch(K.iter_exec, st));
     ctx->launches += K.iter_nodes;
+    return 0;
+}
+
+extern "C" int hemo_krylov_graph_info(hemo_ctx* ctx, int64_t* kernel_nodes, int64_t* programmatic_edges) {
+    if (!ctx || !kernel_nodes || !programmatic_edges) return HEMO_EINVAL;
+    if (!ctx->kry.iter_valid) HEMO_FAIL(ctx, HEMO_ESTATE, "no FGMRES iteration graph has been captured");
+    *kernel_nodes = ctx->kry.iter_kernel_nodes;
+    *programmatic_edges = ctx->kry.iter_prog_edges;
     return 0;
 }
 

@@ -201,6 +201,8 @@ k_bsr_spmv(int n, const int32_t* __restrict__ rowptr, const int32_t* __restrict_
     const int lane = gt & 3;
     const bool ok = i < n;
     const int r0 = ok ? rowptr[i] : 0, r1 = ok ? rowptr[i + 1] : 0;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double a0 = 0.0, a1 = 0.0;
     // column loads of three strided entries first (the col -> x chain bounds short rows)
     for (int t = r0 + lane; t < r1; t += 12) {
@@ -249,9 +251,8 @@ k_bsr_spmv(int n, const int32_t* __restrict__ rowptr, const int32_t* __restrict_
 int hemo_bsr_spmv_ex(hemo_ctx* ctx, int bs, int n, const int32_t* rowptr, const int32_t* col, const areal* val,
                      const areal* x, double alpha, const areal* b, areal* y) {
     const int grid = hemo_grid((int64_t)n * 4, 256);
-    if (bs == 1) k_bsr_spmv<1><<<grid, 256, 0, ctx->stream>>>(n, rowptr, col, val, x, alpha, b, y);
-    else k_bsr_spmv<2><<<grid, 256, 0, ctx->stream>>>(n, rowptr, col, val, x, alpha, b, y);
-    HEMO_LAUNCH_CHECK(ctx);
+    if (bs == 1) HEMO_LAUNCH(ctx, k_bsr_spmv<1>, grid, 256, 0, ctx->stream, n, rowptr, col, val, x, alpha, b, y);
+    else HEMO_LAUNCH(ctx, k_bsr_spmv<2>, grid, 256, 0, ctx->stream, n, rowptr, col, val, x, alpha, b, y);
     return 0;
 }
 
@@ -503,6 +504,8 @@ __global__ void __launch_bounds__(RED_THREADS)
 k_sub_mean_partials(int64_t n, int nparts, const double* __restrict__ partial, double* __restrict__ x) {
     __shared__ double sh[32];
     __shared__ double mean;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc = 0.0;
     for (int t = threadIdx.x; t < nparts; t += blockDim.x) acc += partial[t];
     acc = block_sum(acc, sh);
@@ -517,6 +520,8 @@ k_sub_mean_partials(int64_t n, int nparts, const double* __restrict__ partial, d
 __global__ void __launch_bounds__(RED_THREADS)
 k_sum_partial(int64_t n, const double* src, double* dst, double* __restrict__ partial) {
     __shared__ double sh[32];
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double acc = 0.0;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const double v = src[i];
@@ -532,10 +537,8 @@ int hemo_copy_remove_mean(hemo_ctx* ctx, int64_t n, const double* src, double* x
     int rc = hemo_ensure_reduce(ctx, (size_t)RED_BLOCKS * 2, 512);
     if (rc) return rc;
     const int g = grid_for(n);
-    k_sum_partial<<<g, RED_THREADS, 0, ctx->stream>>>(n, src, x, ctx->red_partial);
-    HEMO_LAUNCH_CHECK(ctx);
-    k_sub_mean_partials<<<g, RED_THREADS, 0, ctx->stream>>>(n, g, ctx->red_partial, x);
-    HEMO_LAUNCH_CHECK(ctx);
+    HEMO_LAUNCH(ctx, k_sum_partial, g, RED_THREADS, 0, ctx->stream, n, src, x, ctx->red_partial);
+    HEMO_LAUNCH(ctx, k_sub_mean_partials, g, RED_THREADS, 0, ctx->stream, n, g, ctx->red_partial, x);
     return 0;
 }
 

@@ -9,6 +9,7 @@
 // Parity with the reference is therefore on the converged solution, never on
 // iteration counts.
 #include <math.h>
+#include <stdlib.h>
 
 #include "hemo_internal.cuh"
 
@@ -87,7 +88,10 @@ __global__ void k_areal_to_double(int64_t n, const areal* __restrict__ x, double
 // x[node*bs + k] = 0 on masked nodes
 __global__ void k_mask_nodes(int n, int bs, const uint8_t* __restrict__ mask, double* __restrict__ x) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || !mask[i]) return;
+    const bool masked = i < n && mask[i];
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
+    if (!masked) return;
     for (int k = 0; k < bs; ++k) x[(int64_t)i * bs + k] = 0.0;
 }
 
@@ -100,10 +104,17 @@ k_a01_residual(int n, const int32_t* __restrict__ nrowptr, const int32_t* __rest
     const int i = gt >> 2, lane = gt & 3;
     const bool ok = i < n;
     const int r0 = ok ? nrowptr[i] : 0, r1 = ok ? nrowptr[i + 1] : 0;
+    // first entry of the lane (constant during the solve) before the wait
+    areal2 g;
+    g.x = g.y = 0;
+    int c = 0;
+    if (r0 + lane < r1) { g = a01[r0 + lane]; c = ncol[r0 + lane]; }
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double a0 = 0.0, a1 = 0.0;
     for (int s = r0 + lane; s < r1; s += 4) {
-        const areal2 g = a01[s];
-        const double z = zp[ncol[s]];
+        if (s != r0 + lane) { g = a01[s]; c = ncol[s]; }
+        const double z = zp[c];
         a0 = fma((double)g.x, z, a0);
         a1 = fma((double)g.y, z, a1);
     }
@@ -125,19 +136,28 @@ k_a01_residual_row(int n, const int32_t* __restrict__ nrowptr, const int32_t* __
                    const areal2* __restrict__ a01, const double* __restrict__ zp, const double* __restrict__ ru,
                    double* __restrict__ tu) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const int r0 = nrowptr[i], r1 = nrowptr[i + 1];
-    double a0 = 0.0, a1 = 0.0;
-    for (int s = r0; s < r1; s += 4) {
-        int t[4], j[4];
-        areal2 g[4];
-        double z[4];
+    const bool ok = i < n;
+    const int r0 = ok ? nrowptr[i] : 0, r1 = ok ? nrowptr[i + 1] : 0;
+    int j[4];
+    areal2 g[4];
+    // column indices and A01 entries of the first four (constant during the solve) before the wait
+    auto fetch = [&](int s) {
+        int t[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) t[u] = s + u < r1 ? s + u : r1 - 1;
 #pragma unroll
         for (int u = 0; u < 4; ++u) j[u] = ncol[t[u]];
 #pragma unroll
         for (int u = 0; u < 4; ++u) g[u] = a01[t[u]];
+    };
+    if (r0 < r1) fetch(r0);
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
+    if (!ok) return;
+    double a0 = 0.0, a1 = 0.0;
+    for (int s = r0; s < r1; s += 4) {
+        double z[4];
+        if (s != r0) fetch(s);
         __syncwarp(__activemask());
 #pragma unroll
         for (int u = 0; u < 4; ++u) z[u] = zp[j[u]];
@@ -161,6 +181,8 @@ k_node_spmv_scalar(int n, const int32_t* __restrict__ nrowptr, const int32_t* __
     const int i = gt >> 2, lane = gt & 3;
     const bool ok = i < n;
     const int r0 = ok ? nrowptr[i] : 0, r1 = ok ? nrowptr[i + 1] : 0;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     double a = 0.0;
     for (int s = r0 + lane; s < r1; s += 4) a = fma((double)val[s], q[ncol[s]], a);
     a += __shfl_down_sync(0xffffffffu, a, 2, 4);
@@ -174,6 +196,8 @@ __global__ void k_schur_combine(int n, double cm, double cl, double cc, const do
                                 const double* __restrict__ conv, const uint8_t* __restrict__ dofflag /* pressure part, n */,
                                 const double* __restrict__ rp, double* __restrict__ zp) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
     if (i >= n) return;
     double v = cm * tp[i] / mass[i] + cl * qp[i];
     if (conv) v += cc * conv[i] / mass[i];
@@ -262,9 +286,11 @@ static int coarse_pressure_fork(hemo_ctx* ctx, const double* t_dev) {
         if ((rc = hemo_comm_allreduce_j(ctx, ctx->coarse_rhs, nc))) break;
         cudaStream_t saved = cc->stream;
         const bool saved_cap = cc->capturing;
+        const int saved_pdl = cc->pdl;
         const int64_t before = cc->launches;
         cc->stream = side;
         cc->capturing = ctx->capturing;
+        cc->pdl = ctx->pdl;
         cc->opts.cheb_degree = ctx->opts.cheb_degree;
         cc->opts.cheb_degree_pre = ctx->opts.cheb_degree_pre;
         cc->opts.cheb_ratio = ctx->opts.cheb_ratio;
@@ -272,6 +298,7 @@ static int coarse_pressure_fork(hemo_ctx* ctx, const double* t_dev) {
         ctx->launches += cc->launches - before;
         cc->stream = saved;
         cc->capturing = saved_cap;
+        cc->pdl = saved_pdl;
         if (rc) ctx->err = cc->err;
     } while (0);
     ctx->stream = main_st;
@@ -491,10 +518,7 @@ int hemo_pc_apply_body(hemo_ctx* ctx, const double* vals_dev, const double* r_de
         if ((rc = hemo_copy_remove_mean(ctx, n, rp, tp))) return rc;      // the copy rides on the summation pass
     } else {
         HEMO_CHECK_CUDA(ctx, cudaMemcpyAsync(tp, rp, sizeof(double) * n, cudaMemcpyDeviceToDevice, st));
-        if (ctx->pc_mask) {
-            k_mask_nodes<<<hemo_grid(n, 256), 256, 0, st>>>(n, 1, ctx->pc_mask, tp);
-            HEMO_LAUNCH_CHECK(ctx);
-        }
+        if (ctx->pc_mask) HEMO_LAUNCH(ctx, k_mask_nodes, hemo_grid(n, 256), 256, 0, st, n, 1, ctx->pc_mask, tp);
         if (ctx->opts.project_pressure && (rc = hemo_remove_mean(ctx, n, tp))) return rc;
     }
     if (ctx->coarse_ctx && (rc = coarse_pressure_fork(ctx, tp))) return rc;
@@ -507,28 +531,22 @@ int hemo_pc_apply_body(hemo_ctx* ctx, const double* vals_dev, const double* r_de
     const bool pcd = ctx->npconv_coef != 0.0 && ctx->npconv;
     if (pcd) {
         // pressure convection-diffusion term: S^-1 ~ 2 Mp^-1 Fp Lp^-1 with Fp = rho/dt Mp + rho/2 Np + mu/2 Lp
-        k_node_spmv_scalar<<<hemo_grid((int64_t)n * 4, 256), 256, 0, st>>>(n, ctx->nrowptr, ctx->ncol, ctx->npconv, qp,
-                                                                          ctx->pc_tmp_u2);
-        HEMO_LAUNCH_CHECK(ctx);
+        HEMO_LAUNCH(ctx, k_node_spmv_scalar, hemo_grid((int64_t)n * 4, 256), 256, 0, st, n, ctx->nrowptr, ctx->ncol, ctx->npconv,
+                    qp, ctx->pc_tmp_u2);
     }
-    k_schur_combine<<<hemo_grid(n, 256), 256, 0, st>>>(n, ctx->opts.schur_mass_coef, ctx->opts.schur_lap_coef,
-                                                       ctx->npconv_coef, tp, ctx->mass, qp,
-                                                       pcd ? ctx->pc_tmp_u2 : nullptr, pressure_flags(ctx), rp, zp);
-    HEMO_LAUNCH_CHECK(ctx);
+    HEMO_LAUNCH(ctx, k_schur_combine, hemo_grid(n, 256), 256, 0, st, n, ctx->opts.schur_mass_coef, ctx->opts.schur_lap_coef,
+                ctx->npconv_coef, tp, ctx->mass, qp, pcd ? ctx->pc_tmp_u2 : nullptr, pressure_flags(ctx), rp, zp);
     if (ctx->opts.project_pressure && (rc = hemo_remove_mean(ctx, n, zp))) return rc;
     }   // else: z_p was provided by the caller (global pressure solve of the multi-GPU driver)
     if (ctx->dim == 3)    // t_u = r_u - A01 z_p, then damped block-Jacobi sweeps on A00 (amg_cycles_u * 4 sweeps)
         return hemo_tet_velocity_solve(ctx, vals_dev, ru, zp, tu, ctx->pc_tmp_u2, zu, 4 * ctx->opts.amg_cycles_u, 2.0 / 3.0);
     // t_u = r_u - A01 z_p
     if (n >= 32768 && ctx->nnz_node <= 12 * (int64_t)n)
-        k_a01_residual_row<<<hemo_grid(n, 256), 256, 0, st>>>(n, ctx->nrowptr, ctx->ncol, ctx->a01, zp, ru, tu);
+        HEMO_LAUNCH(ctx, k_a01_residual_row, hemo_grid(n, 256), 256, 0, st, n, ctx->nrowptr, ctx->ncol, ctx->a01, zp, ru, tu);
     else
-        k_a01_residual<<<hemo_grid((int64_t)n * 4, 256), 256, 0, st>>>(n, ctx->nrowptr, ctx->ncol, ctx->a01, zp, ru, tu);
-    HEMO_LAUNCH_CHECK(ctx);
-    if (ctx->pc_mask) {
-        k_mask_nodes<<<hemo_grid(n, 256), 256, 0, st>>>(n, 2, ctx->pc_mask, tu);
-        HEMO_LAUNCH_CHECK(ctx);
-    }
+        HEMO_LAUNCH(ctx, k_a01_residual, hemo_grid((int64_t)n * 4, 256), 256, 0, st, n, ctx->nrowptr, ctx->ncol, ctx->a01, zp, ru,
+                    tu);
+    if (ctx->pc_mask) HEMO_LAUNCH(ctx, k_mask_nodes, hemo_grid(n, 256), 256, 0, st, n, 2, ctx->pc_mask, tu);
     if ((rc = hemo_amg_vcycle(ctx, &ctx->amg[0], tu, zu, ctx->opts.amg_cycles_u))) return rc;
     return 0;
 }
@@ -622,6 +640,8 @@ extern "C" int hemo_ctx_create(int device, hemo_ctx** out) {
     ctx->opts.schur_lap_coef = 1.0;
     ctx->opts.cheb_ratio = 4.0;
     ctx->opts.cheb_degree_pre = 0;
+    const char* pdl = getenv("HEMO_PDL");
+    ctx->pdl = pdl && atoi(pdl) == 0 ? 0 : 1;
     *out = ctx;
     return 0;
 }

@@ -374,6 +374,10 @@ int hemo_pc_apply(hemo_ctx* ctx, const double* vals_dev, const double* r_dev, do
  * host.  With a communicator (hemo_comm_init) b and y are local vectors; y returns with valid ghosts. */
 int hemo_fgmres(hemo_ctx* ctx, const double* vals_dev, const double* b_dev, double* y_dev,
                 int* its_out, double* rel_resid_out);
+/* Kernel nodes and programmatic-dependent-launch edges of the most recently captured FGMRES iteration
+ * graph (HEMO_PDL=0 in the environment at hemo_ctx_create launches every kernel plainly: no such edges).
+ * HEMO_ESTATE before the first graph has been captured. */
+int hemo_krylov_graph_info(hemo_ctx* ctx, int64_t* kernel_nodes, int64_t* programmatic_edges);
 
 #ifdef __cplusplus
 }
