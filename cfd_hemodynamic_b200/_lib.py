@@ -18,6 +18,8 @@ LIB_PATH = os.path.join(_HERE, "libhemo_sm100.so")
 HEMO_DIVERGED = -100
 Q_FU, Q_FP, Q_UU, Q_UP, Q_PU, Q_PP = range(6)
 CELL_TRIANGLE, CELL_QUADRILATERAL, CELL_TETRAHEDRON, CELL_TRIANGLE_P2 = 0, 1, 2, 3
+# hemo_amg_level_info: what runs an AMG level
+AMG_SCOPE_NAMES = ("level", "cta", "grid", "cluster", "dense")
 
 
 class HemoError(RuntimeError):
@@ -105,6 +107,7 @@ SYMBOLS = {
     "hemo_pc_setup": (_I, [_VP, _VP, _VP, _VP]),
     "hemo_amg_apply": (_I, [_VP, _I, _VP, _VP, _I]),
     "hemo_amg_get_level_values": (_I, [_VP, _I, _I, _VP, _L]),
+    "hemo_amg_level_info": (_I, [_VP, _I, _I, C.POINTER(_L)]),
     "hemo_pc_apply": (_I, [_VP, _VP, _VP, _VP]),
     "hemo_fgmres": (_I, [_VP, _VP, _VP, _VP, C.POINTER(_I), C.POINTER(_D)]),
     "hemo_comm_unique_id": (_I, [C.c_char_p]),
@@ -460,6 +463,14 @@ class Hemo:
         self._check(self.lib.hemo_amg_get_level_values(self._ctx, which, level, _ptr(out), count),
                     "hemo_amg_get_level_values")
         return out
+
+    def amg_level_info(self, which, level):
+        """dict(n, nnzb, sell, scope) of level `level` of hierarchy `which`: sell = entries of the sliced-ELL copy
+        (0: CSR kernels); scope = "level" (per-level kernels), "cta" / "grid" / "cluster" (fused coarse V-cycle
+        kernels) or "dense" (coarsest-level solve)."""
+        out = (C.c_int64 * 4)()
+        self._check(self.lib.hemo_amg_level_info(self._ctx, which, level, out), "hemo_amg_level_info")
+        return dict(n=out[0], nnzb=out[1], sell=out[2], scope=AMG_SCOPE_NAMES[out[3]])
 
     def pc_apply(self, vals, r, z):
         self._check(self.lib.hemo_pc_apply(self._ctx, _ptr(vals), _ptr(r), _ptr(z)), "hemo_pc_apply")

@@ -1020,16 +1020,17 @@ __device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const ar
 
 template <int BS, typename Scope>
 __device__ void coarse_vcycle_body(const Scope& sc, const HemoCoarseLevel* __restrict__ desc, int nl,
-                                   const areal* __restrict__ b0, areal* __restrict__ x0, int degree_pre, int degree,
-                                   double ratio, const double* __restrict__ dense_inv, int dense_n) {
+                                   const areal* __restrict__ b0, areal* __restrict__ x0, int x0_is_zero, int degree_pre,
+                                   int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
     const int tid = sc.tid(), T = sc.nthreads();
     // down sweep
     for (int l = 0; l + 1 < nl; ++l) {
         const HemoCoarseLevel L = desc[l];
         const areal* b = (l == 0) ? b0 : L.b;
         areal* x = (l == 0) ? x0 : L.x;
-        // the levels small enough for one CTA keep the stronger pre-smoother they have always had
-        fused_smooth<BS>(sc, L, b, x, true, L.n <= HEMO_FUSE_STRONG_PRE_NODES ? degree : degree_pre, ratio);
+        // the levels small enough for one CTA keep the stronger pre-smoother they have always had; the top level of a
+        // second or later cycle smooths its previous iterate, every coarser level starts from zero
+        fused_smooth<BS>(sc, L, b, x, l > 0 || x0_is_zero, L.n <= HEMO_FUSE_STRONG_PRE_NODES ? degree : degree_pre, ratio);
         rows_matvec<BS>(sc, L, x, [&](int i, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) L.r[i * BS + k] = (areal)((double)b[i * BS + k] - acc[k]);
@@ -1078,27 +1079,27 @@ __device__ void coarse_vcycle_body(const Scope& sc, const HemoCoarseLevel* __res
 template <int BS>
 __global__ void __launch_bounds__(1024)
 k_coarse_vcycle(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
+                int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
     hemo_pdl_wait();
     hemo_pdl_trigger();
     CtaScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, degree_pre, degree, ratio, dense_inv, dense_n);
+    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
 }
 
 template <int BS>
 __global__ void __launch_bounds__(1024)
 k_coarse_vcycle_cluster(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                        int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
+                        int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
     ClusterScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, degree_pre, degree, ratio, dense_inv, dense_n);
+    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
 }
 
 template <int BS>
 __global__ void __launch_bounds__(512)
 k_coarse_vcycle_grid(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                     int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
+                     int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
     GridScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, degree_pre, degree, ratio, dense_inv, dense_n);
+    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
 }
 
 // ---------------------------------------------------------------------------
@@ -1580,10 +1581,11 @@ static int vcycle_t(hemo_ctx* ctx, HemoAmg* amg, int l, const areal* b, areal* x
     if (l == amg->fuse_level_grid && amg->grid_blocks > 0) {
         // every remaining level inside one persistent cooperative kernel
         const HemoCoarseLevel* desc = amg->fuse_desc + (l - amg->fuse_base);
-        int nl = amg->nlev - l, dp = degree_pre, dg = degree, dn = amg->dense_n;
+        int nl = amg->nlev - l, xz = x_is_zero ? 1 : 0, dp = degree_pre, dg = degree, dn = amg->dense_n;
         double rt = ratio;
         const double* dinv = amg->dense_inv;
-        void* args[] = {(void*)&desc, (void*)&nl, (void*)&b, (void*)&x, (void*)&dp, (void*)&dg, (void*)&rt, (void*)&dinv, (void*)&dn};
+        void* args[] = {(void*)&desc, (void*)&nl, (void*)&b, (void*)&x, (void*)&xz, (void*)&dp, (void*)&dg, (void*)&rt,
+                        (void*)&dinv, (void*)&dn};
         const void* fn = (BS == 2) ? (const void*)k_coarse_vcycle_grid<2> : (const void*)k_coarse_vcycle_grid<1>;
         cudaError_t e = cudaLaunchCooperativeKernel(fn, dim3(amg->grid_blocks), dim3(512), args, 0, st);
         if (e == cudaSuccess) {
@@ -1605,15 +1607,15 @@ static int vcycle_t(hemo_ctx* ctx, HemoAmg* amg, int l, const areal* b, areal* x
         cfg.attrs = at; cfg.numAttrs = 1;
         const HemoCoarseLevel* desc = amg->fuse_desc + (l - amg->fuse_base);
         const double* dinv = amg->dense_inv;
-        HEMO_CHECK_CUDA(ctx, cudaLaunchKernelEx(&cfg, k_coarse_vcycle_cluster<BS>, desc, amg->nlev - l, b, x, degree_pre, degree,
-                                                ratio, dinv, amg->dense_n));
+        HEMO_CHECK_CUDA(ctx, cudaLaunchKernelEx(&cfg, k_coarse_vcycle_cluster<BS>, desc, amg->nlev - l, b, x, x_is_zero ? 1 : 0,
+                                                degree_pre, degree, ratio, dinv, amg->dense_n));
         ctx->launches++;
         return 0;
     }
     if (l == amg->fuse_level) {
         // every remaining level fits one CTA
-        HEMO_LAUNCH(ctx, k_coarse_vcycle<BS>, 1, 1024, 0, st, amg->fuse_desc + (l - amg->fuse_base), amg->nlev - l, b, x, degree_pre,
-                    degree, ratio, amg->dense_inv, amg->dense_n);
+        HEMO_LAUNCH(ctx, k_coarse_vcycle<BS>, 1, 1024, 0, st, amg->fuse_desc + (l - amg->fuse_base), amg->nlev - l, b, x,
+                    x_is_zero ? 1 : 0, degree_pre, degree, ratio, amg->dense_inv, amg->dense_n);
         return 0;
     }
     if (l == amg->nlev - 1) {

@@ -403,7 +403,20 @@ extern "C" int hemo_use_graph(hemo_ctx* ctx, int on) {
 extern "C" int hemo_set_solver_opts(hemo_ctx* ctx, const hemo_solver_opts* o) {
     if (!ctx || !o) return HEMO_EINVAL;
     if (o->restart < 1 || o->restart > 400 || o->max_it < 1) return HEMO_EINVAL;
+    // fields the captured graphs (FGMRES iteration, preconditioner, hemo_amg_apply) bake in as launch arguments or
+    // launch sequence: a change re-captures them at their next use
+    const hemo_solver_opts& p = ctx->opts;
+    const bool baked = p.amg_cycles_u != o->amg_cycles_u || p.amg_cycles_p != o->amg_cycles_p ||
+                       p.cheb_degree != o->cheb_degree || p.cheb_degree_pre != o->cheb_degree_pre ||
+                       p.cheb_ratio != o->cheb_ratio || p.project_pressure != o->project_pressure ||
+                       p.pc_mode != o->pc_mode || p.schur_mass_coef != o->schur_mass_coef ||
+                       p.schur_lap_coef != o->schur_lap_coef;
     ctx->opts = *o;
+    if (baked) {
+        hemo_krylov_invalidate(ctx);
+        ctx->pc_graph_dirty = true;
+        ctx->amg[0].apply_valid = ctx->amg[1].apply_valid = false;
+    }
     return 0;
 }
 
@@ -499,6 +512,25 @@ extern "C" int hemo_amg_get_level_values(hemo_ctx* ctx, int which, int level, do
     if (capacity < cnt) return HEMO_EINVAL;
     k_areal_to_double<<<hemo_grid(cnt, 256), 256, 0, ctx->stream>>>(cnt, amg.op[level].val, vals_dev);
     HEMO_LAUNCH_CHECK(ctx);
+    return 0;
+}
+
+extern "C" int hemo_amg_level_info(hemo_ctx* ctx, int which, int level, int64_t* out) {
+    if (!ctx || which < 0 || which > 1 || !out) return HEMO_EINVAL;
+    const HemoAmg& amg = ctx->amg[which];
+    if (!amg.ready || level < 0 || level >= amg.nlev) return HEMO_EINVAL;
+    const HemoAmgOp& o = amg.op[level];
+    // the order of the tests follows vcycle_t: a level runs in the first fused kernel whose range covers it; the grid
+    // kernel counts only while its cooperative launch is available (grid_blocks drops to 0 when it fails)
+    int scope = HEMO_AMG_SCOPE_LEVEL;
+    if (amg.grid_blocks > 0 && amg.fuse_level_grid >= 0 && level >= amg.fuse_level_grid) scope = HEMO_AMG_SCOPE_GRID;
+    else if (amg.cluster_ctas > 0 && amg.fuse_level_cluster >= 0 && level >= amg.fuse_level_cluster) scope = HEMO_AMG_SCOPE_CLUSTER;
+    else if (amg.fuse_level >= 0 && level >= amg.fuse_level) scope = HEMO_AMG_SCOPE_CTA;
+    else if (level == amg.nlev - 1) scope = HEMO_AMG_SCOPE_DENSE;
+    out[0] = o.n;
+    out[1] = o.nnzb;
+    out[2] = o.sell_ptr ? o.sell_entries : 0;
+    out[3] = scope;
     return 0;
 }
 

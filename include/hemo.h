@@ -264,6 +264,8 @@ int hemo_host_aggregate(int n, const int32_t* rowptr, const int32_t* col, const 
                         int32_t* agg, int32_t* n_agg_out);
 
 /* ---- solve ------------------------------------------------------------------------ */
+/* Takes effect at the next hemo_pc_apply / hemo_amg_apply / hemo_fgmres: a change of the cycles, Chebyshev
+ * parameters, Schur coefficients, project_pressure or pc_mode re-captures the graphs that bake them in. */
 int hemo_set_solver_opts(hemo_ctx* ctx, const hemo_solver_opts* o);
 /* PCSetUp (pc.setUp(), src/solvers/stabilized_schur.py:253 and every Newton
  * iteration): numeric Galerkin products of the A00 hierarchy from the current
@@ -277,6 +279,14 @@ int hemo_amg_apply(hemo_ctx* ctx, int which, const double* b_dev, double* x_dev,
 /* Level operator of hierarchy `which` after hemo_pc_setup (device copy out;
  * nnzb*bs*bs doubles).  Exposed for the Galerkin-product parity test. */
 int hemo_amg_get_level_values(hemo_ctx* ctx, int which, int level, double* vals_dev, int64_t capacity);
+/* Which kernels run level `level` of hierarchy `which` (read-only, after hemo_amg_finalize):
+ * out[0] = block rows n, out[1] = blocks nnzb, out[2] = entries of the sliced-ELL copy (0: CSR kernels),
+ * out[3] = HEMO_AMG_SCOPE_*: the per-level kernels, one of the fused coarse V-cycle kernels (one CTA,
+ * cooperative grid, thread-block cluster) or the dense coarsest-level solve.  Read at the time of the
+ * call: the grid scope falls back to the others once a cooperative launch has failed. */
+enum { HEMO_AMG_SCOPE_LEVEL = 0, HEMO_AMG_SCOPE_CTA = 1, HEMO_AMG_SCOPE_GRID = 2, HEMO_AMG_SCOPE_CLUSTER = 3,
+       HEMO_AMG_SCOPE_DENSE = 4 };
+int hemo_amg_level_info(hemo_ctx* ctx, int which, int level, int64_t out[4]);
 /* ---- multi-GPU building blocks (domain decomposition, one partition per GPU) ----------
  * The host driver (cfd_hemodynamic_b200/parallel.py) exchanges ghost values and sums the
  * Krylov reductions with torch.distributed (NCCL); these entry points are the local,
