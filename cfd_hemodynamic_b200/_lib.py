@@ -19,7 +19,7 @@ HEMO_DIVERGED = -100
 Q_FU, Q_FP, Q_UU, Q_UP, Q_PU, Q_PP = range(6)
 CELL_TRIANGLE, CELL_QUADRILATERAL, CELL_TETRAHEDRON, CELL_TRIANGLE_P2 = 0, 1, 2, 3
 # hemo_amg_level_info: what runs an AMG level
-AMG_SCOPE_NAMES = ("level", "cta", "grid", "cluster", "dense")
+AMG_SCOPE_NAMES = ("level", "cta")
 
 
 class HemoError(RuntimeError):
@@ -99,11 +99,8 @@ SYMBOLS = {
     "hemo_vec_maxpy": (_I, [_VP, _L, _I, _VP, _L, _VP, _D, _VP, C.POINTER(_D)]),
     "hemo_vec_scale": (_I, [_VP, _L, _D, _VP, _VP]),
     "hemo_use_graph": (_I, [_VP, _I]),
-    "hemo_set_schur_mask": (_I, [_VP, _VP]),
-    "hemo_pc_set_schur_operator": (_I, [_VP, _VP, _VP, _VP, _D, _D]),
     "hemo_amg_set_fine_pattern": (_I, [_VP, _I, _VP, _VP]),
     "hemo_pc_set_schur_selfp": (_I, [_VP, _VP, _D]),
-    "hemo_pc_set_convection": (_I, [_VP, _VP, _VP, _D]),
     "hemo_pc_setup": (_I, [_VP, _VP, _VP, _VP]),
     "hemo_amg_apply": (_I, [_VP, _I, _VP, _VP, _I]),
     "hemo_amg_get_level_values": (_I, [_VP, _I, _I, _VP, _L]),
@@ -425,14 +422,6 @@ class Hemo:
     def use_graph(self, on: bool):
         self._check(self.lib.hemo_use_graph(self._ctx, int(on)), "hemo_use_graph")
 
-    def set_schur_mask(self, node_mask):
-        self._check(self.lib.hemo_set_schur_mask(self._ctx, _ptr(node_mask)), "hemo_set_schur_mask")
-
-    def pc_set_schur_operator(self, x, un, vals, c_u=1.0, coarse_shift=0.0):
-        self._check(self.lib.hemo_pc_set_schur_operator(self._ctx, _ptr(x), _ptr(un), _ptr(vals), float(c_u),
-                                                        float(coarse_shift)),
-                    "hemo_pc_set_schur_operator")
-
     def amg_set_fine_pattern(self, which, pattern):
         """pattern: scipy CSR (values ignored) or None to fall back to the node graph."""
         if pattern is None:
@@ -445,9 +434,6 @@ class Hemo:
 
     def pc_set_schur_selfp(self, vals, coarse_shift=0.0):
         self._check(self.lib.hemo_pc_set_schur_selfp(self._ctx, _ptr(vals), float(coarse_shift)), "hemo_pc_set_schur_selfp")
-
-    def pc_set_convection(self, x, un, coef):
-        self._check(self.lib.hemo_pc_set_convection(self._ctx, _ptr(x), _ptr(un), float(coef)), "hemo_pc_set_convection")
 
     def pc_setup(self, vals, lap=None, mass=None):
         if lap is not None:
@@ -466,8 +452,7 @@ class Hemo:
 
     def amg_level_info(self, which, level):
         """dict(n, nnzb, sell, scope) of level `level` of hierarchy `which`: sell = entries of the sliced-ELL copy
-        (0: CSR kernels); scope = "level" (per-level kernels), "cta" / "grid" / "cluster" (fused coarse V-cycle
-        kernels) or "dense" (coarsest-level solve)."""
+        (0: CSR kernels); scope = "level" (per-level kernels) or "cta" (the one-CTA fused coarse V-cycle kernel)."""
         out = (C.c_int64 * 4)()
         self._check(self.lib.hemo_amg_level_info(self._ctx, which, level, out), "hemo_amg_level_info")
         return dict(n=out[0], nnzb=out[1], sell=out[2], scope=AMG_SCOPE_NAMES[out[3]])

@@ -10,7 +10,6 @@
 // mesh graph and are built once by the host; what runs here every Newton
 // iteration is the numeric Galerkin product R*A*P on fixed patterns, the
 // smoother set-up, and the cycles.
-#include <cooperative_groups.h>
 #include <type_traits>
 #include <cub/device/device_scan.cuh>
 
@@ -20,7 +19,9 @@ int hemo_bsr_spmv_ex(hemo_ctx* ctx, int bs, int n, const int32_t* rowptr, const 
                      const areal* x, double alpha, const areal* b, areal* y);
 
 // ---------------------------------------------------------------------------
-// numeric Galerkin product
+// Numeric Galerkin product through precomputed gather lists: one thread per
+// output block, contributions summed in a fixed order, no searches at run time.
+// The lists are built once on the device.
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ int find_col(const int32_t* __restrict__ col, int lo, int hi, int key) {
     // binary search in col[lo, hi)
@@ -34,89 +35,6 @@ __device__ __forceinline__ int find_col(const int32_t* __restrict__ col, int lo,
     return -1;
 }
 
-// AP = A * (P (x) I_bs): 8 lanes per fine block row; each lane owns one output
-// block of the row and scans the (A entry, P entry) pairs — no searches, no
-// read-modify-write on global memory, fixed summation order.
-template <int BS>
-__global__ void __launch_bounds__(256)
-k_numeric_ap(int n, const int32_t* __restrict__ a_rowptr, const int32_t* __restrict__ a_col,
-             const areal* __restrict__ a_val, const int32_t* __restrict__ p_rowptr,
-             const int32_t* __restrict__ p_col, const double* __restrict__ p_val,
-             const int32_t* __restrict__ ap_rowptr, const int32_t* __restrict__ ap_col,
-             areal* __restrict__ ap_val) {
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = gt >> 3, lane = gt & 7;
-    if (i >= n) return;
-    const int o0 = ap_rowptr[i], o1 = ap_rowptr[i + 1];
-    const int t0 = a_rowptr[i], t1 = a_rowptr[i + 1];
-    for (int base = o0; base < o1; base += 8) {
-        const int s = base + lane;
-        const int myc = (s < o1) ? ap_col[s] : -1;
-        double acc[BS * BS];
-#pragma unroll
-        for (int k = 0; k < BS * BS; ++k) acc[k] = 0.0;
-        for (int t = t0; t < t1; ++t) {
-            const int j = a_col[t];
-            const int u1 = p_rowptr[j + 1];
-            for (int u = p_rowptr[j]; u < u1; ++u) {
-                if (p_col[u] == myc) {
-                    const double w = p_val[u];
-#pragma unroll
-                    for (int k = 0; k < BS * BS; ++k) acc[k] = fma(w, (double)a_val[(int64_t)t * BS * BS + k], acc[k]);
-                }
-            }
-        }
-        if (s < o1) {
-#pragma unroll
-            for (int k = 0; k < BS * BS; ++k) ap_val[(int64_t)s * BS * BS + k] = acc[k];
-        }
-    }
-}
-
-// Ac = (R (x) I_bs) * AP: one warp per coarse block row; each lane owns one
-// output block and scans the (R entry, AP entry) pairs of the row (uniform,
-// broadcast loads) — deterministic, no atomics, no searches.
-template <int BS>
-__global__ void __launch_bounds__(256)
-k_numeric_rap(int nc, const int32_t* __restrict__ r_rowptr, const int32_t* __restrict__ r_col,
-              const double* __restrict__ r_val, const int32_t* __restrict__ ap_rowptr,
-              const int32_t* __restrict__ ap_col, const areal* __restrict__ ap_val,
-              const int32_t* __restrict__ c_rowptr, const int32_t* __restrict__ c_col,
-              areal* __restrict__ c_val) {
-    const int I = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (I >= nc) return;
-    const int o0 = c_rowptr[I], o1 = c_rowptr[I + 1];
-    const int t0 = r_rowptr[I], t1 = r_rowptr[I + 1];
-    for (int base = o0; base < o1; base += 32) {
-        const int s = base + lane;
-        const int myc = (s < o1) ? c_col[s] : -1;
-        double acc[BS * BS];
-#pragma unroll
-        for (int k = 0; k < BS * BS; ++k) acc[k] = 0.0;
-        for (int t = t0; t < t1; ++t) {
-            const int i = r_col[t];
-            const double w = r_val[t];
-            const int u1 = ap_rowptr[i + 1];
-            for (int u = ap_rowptr[i]; u < u1; ++u) {
-                if (ap_col[u] == myc) {
-#pragma unroll
-                    for (int k = 0; k < BS * BS; ++k) acc[k] = fma(w, (double)ap_val[(int64_t)u * BS * BS + k], acc[k]);
-                }
-            }
-        }
-        if (s < o1) {
-#pragma unroll
-            for (int k = 0; k < BS * BS; ++k) c_val[(int64_t)s * BS * BS + k] = acc[k];
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------
-// Galerkin product through precomputed gather lists (hierarchy 0, rebuilt every
-// Newton iteration): one thread per output block, contributions summed in a
-// fixed order, no searches at run time.  The lists are built once on the device.
-// ---------------------------------------------------------------------------
 // count / fill pass over "rows x inner entries x outer entries":
 //   AP:  row i,  t in A-row(i),  u in P-row(a_col[t])  -> slot of p_col[u] in AP-row(i);  src = (u, t)
 //   RAP: row I,  t in R-row(I),  u in AP-row(r_col[t]) -> slot of ap_col[u] in C-row(I);  src = (t, u)
@@ -859,49 +777,15 @@ k_transfer(int nrows, const int32_t* __restrict__ rowptr, const int32_t* __restr
 }
 
 // ---------------------------------------------------------------------------
-// fused coarse V-cycle: every level from `fuse_level` down runs inside ONE kernel, phases separated by a
-// barrier, replacing ~7 launches per level.  Two scopes share the code:
-//   GridScope — a persistent cooperative grid (one CTA per SM, cooperative_groups grid.sync between phases):
-//               the levels below the finest are a few thousand rows each, far too small to fill the GPU from
-//               separate launches (each costs 5-10 us of launch + drain), but still too large for one CTA;
-//   CtaScope  — one CTA with __syncthreads (fallback when a cooperative launch is not possible).
+// fused coarse V-cycle: every level from `fuse_level` down (at most HEMO_FUSE_MAX_NODES nodes each) runs inside ONE
+// CTA, phases separated by __syncthreads, replacing ~7 launches per level.
 // ---------------------------------------------------------------------------
-namespace cg = cooperative_groups;
-
-struct CtaScope {
-    __device__ __forceinline__ int tid() const { return threadIdx.x; }
-    __device__ __forceinline__ int nthreads() const { return blockDim.x; }
-    __device__ __forceinline__ void sync() const { __syncthreads(); }
-};
-struct GridScope {
-    cg::grid_group g;
-    __device__ __forceinline__ GridScope() : g(cg::this_grid()) {}
-    __device__ __forceinline__ int tid() const { return blockIdx.x * blockDim.x + threadIdx.x; }
-    __device__ __forceinline__ int nthreads() const { return gridDim.x * blockDim.x; }
-    __device__ __forceinline__ void sync() const { g.sync(); }
-};
-
-// one thread-block cluster: hardware barrier with release / acquire semantics at cluster scope (global-memory writes of
-// the other CTAs are visible after it)
-struct ClusterScope {
-    unsigned rank, nctas;
-    __device__ __forceinline__ ClusterScope() {
-        asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
-        asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(nctas));
-    }
-    __device__ __forceinline__ int tid() const { return (int)(rank * blockDim.x + threadIdx.x); }
-    __device__ __forceinline__ int nthreads() const { return (int)(nctas * blockDim.x); }
-    __device__ __forceinline__ void sync() const {
-        asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-    }
-};
-
 // Row loops: 8 lanes cooperate on one block row (coarse Galerkin rows hold 20-60 blocks; a thread-serial
 // walk makes every phase a ~50-deep dependent load chain).  All lanes of a warp execute the same number of
 // outer iterations, so full-mask shuffles are legal.
-template <int BS, typename Scope, typename Epi>
-__device__ __forceinline__ void rows_matvec(const Scope& sc, const HemoCoarseLevel& L, const areal* __restrict__ x, Epi epi) {
-    const int lane = sc.tid() & 7, group = sc.tid() >> 3, ngroups = sc.nthreads() >> 3;
+template <int BS, typename Epi>
+__device__ __forceinline__ void rows_matvec(const HemoCoarseLevel& L, const areal* __restrict__ x, Epi epi) {
+    const int lane = threadIdx.x & 7, group = threadIdx.x >> 3, ngroups = blockDim.x >> 3;
     for (int base = 0; base < L.n; base += ngroups) {
         const int i = base + group;
         const bool ok = i < L.n;
@@ -930,11 +814,10 @@ __device__ __forceinline__ void rows_matvec(const Scope& sc, const HemoCoarseLev
 }
 
 // y-rows of a transfer operator (CSR with fp64 weights) applied to a BS-component vector
-template <int BS, typename Scope, typename Epi>
-__device__ __forceinline__ void rows_transfer(const Scope& sc, int nrows, const int32_t* __restrict__ rowptr,
-                                              const int32_t* __restrict__ col, const double* __restrict__ w,
-                                              const areal* __restrict__ x, Epi epi) {
-    const int lane = sc.tid() & 7, group = sc.tid() >> 3, ngroups = sc.nthreads() >> 3;
+template <int BS, typename Epi>
+__device__ __forceinline__ void rows_transfer(int nrows, const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                                              const double* __restrict__ w, const areal* __restrict__ x, Epi epi) {
+    const int lane = threadIdx.x & 7, group = threadIdx.x >> 3, ngroups = blockDim.x >> 3;
     for (int base = 0; base < nrows; base += ngroups) {
         const int i = base + group;
         const bool ok = i < nrows;
@@ -960,10 +843,10 @@ __device__ __forceinline__ void rows_transfer(const Scope& sc, int nrows, const 
     }
 }
 
-template <int BS, typename Scope>
-__device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const areal* __restrict__ b, areal* __restrict__ x,
-                             bool x_is_zero, int degree, double ratio) {
-    const int tid = sc.tid(), T = sc.nthreads();
+template <int BS>
+__device__ void fused_smooth(const HemoCoarseLevel& L, const areal* __restrict__ b, areal* __restrict__ x, bool x_is_zero,
+                             int degree, double ratio) {
+    const int tid = threadIdx.x, T = blockDim.x;
     const int N = L.n * BS;
     const double lmax = *L.lmax, lmin = lmax / ratio;
     const double theta = 0.5 * (lmax + lmin), delta = 0.5 * (lmax - lmin), sigma = theta / delta;
@@ -978,7 +861,7 @@ __device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const ar
             x[q] = (areal)(rv / theta);
         }
     } else {
-        rows_matvec<BS>(sc, L, x, [&](int i, const double* acc) {
+        rows_matvec<BS>(L, x, [&](int i, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) {
                 const int q = i * BS + k;
@@ -988,7 +871,7 @@ __device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const ar
             }
         });
     }
-    sc.sync();
+    __syncthreads();
     bool pending = !x_is_zero;
     for (int s = 1; s < degree; ++s) {
         const double rho_new = 1.0 / (2.0 * sigma - rho);
@@ -996,7 +879,7 @@ __device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const ar
         const areal* dcur = dold;
         areal* dnext = dnew;
         const bool add_old = pending;
-        rows_matvec<BS>(sc, L, dcur, [&](int i, const double* acc) {
+        rows_matvec<BS>(L, dcur, [&](int i, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) {
                 const int q = i * BS + k;
@@ -1007,41 +890,43 @@ __device__ void fused_smooth(const Scope& sc, const HemoCoarseLevel& L, const ar
                 x[q] = (areal)((double)x[q] + (add_old ? (dv + (double)dcur[q]) : dv));
             }
         });
-        sc.sync();
+        __syncthreads();
         pending = false;
         areal* t = dold; dold = dnew; dnew = t;
         rho = rho_new;
     }
     if (pending) {
         for (int q = tid; q < N; q += T) x[q] = (areal)((double)x[q] + (double)dold[q]);
-        sc.sync();
+        __syncthreads();
     }
 }
 
-template <int BS, typename Scope>
-__device__ void coarse_vcycle_body(const Scope& sc, const HemoCoarseLevel* __restrict__ desc, int nl,
-                                   const areal* __restrict__ b0, areal* __restrict__ x0, int x0_is_zero, int degree_pre,
-                                   int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
-    const int tid = sc.tid(), T = sc.nthreads();
+template <int BS>
+__global__ void __launch_bounds__(1024)
+k_coarse_vcycle(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
+                int x0_is_zero, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
+    hemo_pdl_wait();
+    hemo_pdl_trigger();
+    const int tid = threadIdx.x, T = blockDim.x;
     // down sweep
-    for (int l = 0; l + 1 < nl; ++l) {
+    for (int l = 0; l < nl - 1; ++l) {
         const HemoCoarseLevel L = desc[l];
         const areal* b = (l == 0) ? b0 : L.b;
         areal* x = (l == 0) ? x0 : L.x;
-        // the levels small enough for one CTA keep the stronger pre-smoother they have always had; the top level of a
-        // second or later cycle smooths its previous iterate, every coarser level starts from zero
-        fused_smooth<BS>(sc, L, b, x, l > 0 || x0_is_zero, L.n <= HEMO_FUSE_STRONG_PRE_NODES ? degree : degree_pre, ratio);
-        rows_matvec<BS>(sc, L, x, [&](int i, const double* acc) {
+        // every level pre-smooths with the full Chebyshev degree; the top level of a second or later cycle smooths its
+        // previous iterate, every coarser level starts from zero
+        fused_smooth<BS>(L, b, x, l > 0 || x0_is_zero, degree, ratio);
+        rows_matvec<BS>(L, x, [&](int i, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) L.r[i * BS + k] = (areal)((double)b[i * BS + k] - acc[k]);
         });
-        sc.sync();
+        __syncthreads();
         areal* bc = desc[l + 1].b;
-        rows_transfer<BS>(sc, L.nc, L.r_rowptr, L.r_col, L.r_val, L.r, [&](int I, const double* acc) {
+        rows_transfer<BS>(L.nc, L.r_rowptr, L.r_col, L.r_val, L.r, [&](int I, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) bc[I * BS + k] = (areal)acc[k];
         });
-        sc.sync();
+        __syncthreads();
     }
     // coarsest: dense inverse, 8 lanes per row
     {
@@ -1059,7 +944,7 @@ __device__ void coarse_vcycle_body(const Scope& sc, const HemoCoarseLevel* __res
             acc += __shfl_xor_sync(0xffffffffu, acc, 4, 8);
             if (ok && lane == 0) x[row] = (areal)acc;
         }
-        sc.sync();
+        __syncthreads();
     }
     // up sweep
     for (int l = nl - 2; l >= 0; --l) {
@@ -1067,44 +952,18 @@ __device__ void coarse_vcycle_body(const Scope& sc, const HemoCoarseLevel* __res
         const areal* b = (l == 0) ? b0 : L.b;
         areal* x = (l == 0) ? x0 : L.x;
         const areal* xc = desc[l + 1].x;
-        rows_transfer<BS>(sc, L.n, L.p_rowptr, L.p_col, L.p_val, xc, [&](int i, const double* acc) {
+        rows_transfer<BS>(L.n, L.p_rowptr, L.p_col, L.p_val, xc, [&](int i, const double* acc) {
 #pragma unroll
             for (int k = 0; k < BS; ++k) x[i * BS + k] = (areal)((double)x[i * BS + k] + acc[k]);
         });
-        sc.sync();
-        fused_smooth<BS>(sc, L, b, x, false, degree, ratio);
+        __syncthreads();
+        fused_smooth<BS>(L, b, x, false, degree, ratio);
     }
 }
 
-template <int BS>
-__global__ void __launch_bounds__(1024)
-k_coarse_vcycle(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
-    hemo_pdl_wait();
-    hemo_pdl_trigger();
-    CtaScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
-}
-
-template <int BS>
-__global__ void __launch_bounds__(1024)
-k_coarse_vcycle_cluster(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                        int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
-    ClusterScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
-}
-
-template <int BS>
-__global__ void __launch_bounds__(512)
-k_coarse_vcycle_grid(const HemoCoarseLevel* __restrict__ desc, int nl, const areal* __restrict__ b0, areal* __restrict__ x0,
-                     int x0_is_zero, int degree_pre, int degree, double ratio, const double* __restrict__ dense_inv, int dense_n) {
-    GridScope sc;
-    coarse_vcycle_body<BS>(sc, desc, nl, b0, x0, x0_is_zero, degree_pre, degree, ratio, dense_inv, dense_n);
-}
-
 // ---------------------------------------------------------------------------
-// dense coarsest-level solve: explicit inverse by Gauss–Jordan with partial
-// pivoting, one CTA (N <= HEMO_DENSE_MAX)
+// dense inverse of the coarsest level (applied by k_coarse_vcycle): Gauss–Jordan,
+// one CTA (N <= HEMO_DENSE_MAX)
 // ---------------------------------------------------------------------------
 template <int BS>
 __global__ void k_dense_fill(int n, const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
@@ -1163,21 +1022,6 @@ k_dense_invert(int N, const double* __restrict__ Min, double* __restrict__ inv, 
     for (int q = tid; q < total; q += blockDim.x) inv[q] = A[q];
 }
 
-// y = inv * b : one warp per row
-__global__ void __launch_bounds__(256)
-k_dense_gemv(int N, const double* __restrict__ inv, const areal* __restrict__ b, areal* __restrict__ y) {
-    const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    hemo_pdl_wait();
-    hemo_pdl_trigger();
-    double acc = 0.0;
-    if (row < N)
-        for (int c = lane; c < N; c += 32) acc += inv[(int64_t)row * N + c] * b[c];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
-    if (row < N && lane == 0) y[row] = acc;
-}
-
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
@@ -1203,8 +1047,7 @@ void hemo_amg_free(HemoAmg* amg) {
     cudaFree(amg->fine_rowptr); cudaFree(amg->fine_col); cudaFree(amg->fine_rowof);
     amg->fine_rowptr = amg->fine_col = amg->fine_rowof = nullptr; amg->fine_nnz = 0;
     cudaFree(amg->dense_inv); cudaFree(amg->dense_work); cudaFree(amg->fuse_desc); cudaFree(amg->lmax_dev);
-    amg->fuse_desc = nullptr; amg->lmax_dev = nullptr; amg->fuse_level = amg->fuse_level_grid = amg->fuse_level_cluster = amg->fuse_base = -1;
-    amg->grid_blocks = amg->cluster_ctas = 0;
+    amg->fuse_desc = nullptr; amg->lmax_dev = nullptr; amg->fuse_level = -1;
     amg->dense_inv = amg->dense_work = nullptr;
     amg->nlev = 0;
     amg->ready = false;
@@ -1271,12 +1114,6 @@ extern "C" int hemo_amg_set_fine_pattern(hemo_ctx* ctx, int which, const int32_t
     HEMO_CHECK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     amg.fine_nnz = nnz;
     return 0;
-}
-
-static int fuse_max_nodes() {
-    const char* env = getenv("HEMO_FUSE_MAX");
-    const int v = env ? atoi(env) : HEMO_FUSE_MAX_NODES;
-    return v > 0 ? v : HEMO_FUSE_MAX_NODES;
 }
 
 // sliced-ELL pattern of one operator (kept when the padding stays below half of the entries)
@@ -1361,86 +1198,34 @@ extern "C" int hemo_amg_finalize(hemo_ctx* ctx, int which, int n_levels) {
                                      L.c_col, L.nnz_c, &L.c_seg_ptr, &L.c_seg_src))) return rc;
         }
     }
-    // levels handled by the fused kernels: from `fuse_level_grid` down by the cooperative persistent grid, from
-    // `fuse_level` (<= HEMO_FUSE_MAX_NODES nodes) down by one CTA when a cooperative launch is not possible
-    amg.fuse_level = amg.fuse_level_grid = -1;
+    // every level from `fuse_level` down runs inside the one-CTA kernel; the coarsest level always does, as it holds at
+    // most HEMO_DENSE_MAX dofs
+    static_assert(HEMO_DENSE_MAX <= HEMO_FUSE_MAX_NODES, "the coarsest level must fit the one-CTA kernel");
+    amg.fuse_level = -1;
     for (int l = 0; l < n_levels; ++l)
-        if (amg.op[l].n <= fuse_max_nodes()) { amg.fuse_level = l; break; }
-    {
-        int coop = 0, sms = 0;
-        cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
-        const char* env = getenv("HEMO_GRID_FUSE_MAX");
-        const int cap = env ? atoi(env) : HEMO_GRID_FUSE_MAX_NODES;
-        amg.grid_blocks = 0;
-        if (coop && sms > 0 && cap > 0) {
-            int occ = 0;
-            if (bs == 2) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_coarse_vcycle_grid<2>, 512, 0);
-            else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_coarse_vcycle_grid<1>, 512, 0);
-            if (occ >= 1) {
-                amg.grid_blocks = sms;
-                for (int l = 1; l < n_levels; ++l)
-                    if (amg.op[l].n <= cap) { amg.fuse_level_grid = l; break; }
-            }
-        }
-        cudaGetLastError();
-    }
-    amg.fuse_level_cluster = -1;
-    amg.cluster_ctas = 0;
-    {
-        const char* env = getenv("HEMO_CLUSTER_FUSE_MAX");
-        const int cap = env ? atoi(env) : HEMO_CLUSTER_FUSE_MAX_NODES;
-        const char* envc = getenv("HEMO_CLUSTER_CTAS");
-        int want = envc ? atoi(envc) : 16;
-        if (want > 16) want = 16;
-        if (cap > fuse_max_nodes() && want > 1 && amg.fuse_level_grid < 0) {
-            const void* fn = (bs == 2) ? (const void*)k_coarse_vcycle_cluster<2> : (const void*)k_coarse_vcycle_cluster<1>;
-            if (want > 8) cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            for (int c = want; c >= 2 && amg.cluster_ctas == 0; c >>= 1) {
-                cudaLaunchConfig_t cfg = {};
-                cfg.gridDim = dim3(c); cfg.blockDim = dim3(1024);
-                cudaLaunchAttribute at[1];
-                at[0].id = cudaLaunchAttributeClusterDimension;
-                at[0].val.clusterDim.x = c; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-                cfg.attrs = at; cfg.numAttrs = 1;
-                int nclusters = 0;
-                if (cudaOccupancyMaxActiveClusters(&nclusters, fn, &cfg) == cudaSuccess && nclusters >= 1) amg.cluster_ctas = c;
-            }
-            cudaGetLastError();
-            if (amg.cluster_ctas > 0)
-                for (int l = 1; l < n_levels; ++l)
-                    if (amg.op[l].n <= cap) {
-                        if (amg.op[l].n > fuse_max_nodes()) amg.fuse_level_cluster = l;
-                        break;
-                    }
-        }
-    }
-    amg.fuse_base = amg.fuse_level_grid >= 0 ? amg.fuse_level_grid
-                  : (amg.fuse_level_cluster >= 0 ? amg.fuse_level_cluster : amg.fuse_level);
+        if (amg.op[l].n <= HEMO_FUSE_MAX_NODES) { amg.fuse_level = l; break; }
     // the levels that keep per-level kernels get the sliced-ELL copy
-    for (int l = 0; l < (amg.fuse_base >= 0 ? amg.fuse_base : n_levels - 1); ++l)
+    for (int l = 0; l < amg.fuse_level; ++l)
         if ((rc = build_sell(ctx, amg.op[l], bs))) return rc;
-    if (amg.fuse_base >= 0) {
-        std::vector<HemoCoarseLevel> d;
-        for (int l = amg.fuse_base; l < n_levels; ++l) {
-            const HemoAmgOp& o = amg.op[l];
-            HemoCoarseLevel c{};
-            c.n = o.n; c.rowptr = o.rowptr; c.col = o.col; c.val = o.val; c.dinv = o.dinv;
-            c.x = o.x; c.b = o.b; c.r = o.r; c.d0 = o.d; c.d1 = o.d + (size_t)o.n * bs;
-            c.lmax = amg.lmax_dev + l;
-            if (l + 1 < n_levels) {
-                const HemoAmgLevel& L = amg.lev[l];
-                c.nc = L.n_coarse;
-                c.p_rowptr = L.p_rowptr; c.p_col = L.p_col; c.p_val = L.p_val;
-                c.r_rowptr = L.r_rowptr; c.r_col = L.r_col; c.r_val = L.r_val;
-            }
-            d.push_back(c);
+    std::vector<HemoCoarseLevel> d;
+    for (int l = amg.fuse_level; l < n_levels; ++l) {
+        const HemoAmgOp& o = amg.op[l];
+        HemoCoarseLevel c{};
+        c.n = o.n; c.rowptr = o.rowptr; c.col = o.col; c.val = o.val; c.dinv = o.dinv;
+        c.x = o.x; c.b = o.b; c.r = o.r; c.d0 = o.d; c.d1 = o.d + (size_t)o.n * bs;
+        c.lmax = amg.lmax_dev + l;
+        if (l + 1 < n_levels) {
+            const HemoAmgLevel& L = amg.lev[l];
+            c.nc = L.n_coarse;
+            c.p_rowptr = L.p_rowptr; c.p_col = L.p_col; c.p_val = L.p_val;
+            c.r_rowptr = L.r_rowptr; c.r_col = L.r_col; c.r_val = L.r_val;
         }
-        if ((rc = hemo_alloc(ctx, &amg.fuse_desc, d.size()))) return rc;
-        HEMO_CHECK_CUDA(ctx, cudaMemcpyAsync(amg.fuse_desc, d.data(), sizeof(HemoCoarseLevel) * d.size(),
-                                             cudaMemcpyHostToDevice, ctx->stream));
-        HEMO_CHECK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        d.push_back(c);
     }
+    if ((rc = hemo_alloc(ctx, &amg.fuse_desc, d.size()))) return rc;
+    HEMO_CHECK_CUDA(ctx, cudaMemcpyAsync(amg.fuse_desc, d.data(), sizeof(HemoCoarseLevel) * d.size(), cudaMemcpyHostToDevice,
+                                         ctx->stream));
+    HEMO_CHECK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     amg.ready = true;
     return 0;
 }
@@ -1460,21 +1245,12 @@ static int amg_numeric_t(hemo_ctx* ctx, HemoAmg* amg, double coarse_shift) {
         HemoAmgOp& C = amg->op[l + 1];
         const HemoAmgLevel& L = amg->lev[l];
         if (l == 0) HEMO_PROF_BEGIN(ctx, HEMO_PROF_RAP);
-        if (L.ap_seg_ptr && L.c_seg_ptr) {
-            k_gather_product<BS><<<hemo_grid(L.nnz_ap, 256), 256, 0, st>>>(L.nnz_ap, L.ap_seg_ptr, L.ap_seg_src, L.p_val,
-                                                                            A.val, L.ap_val);
-            HEMO_LAUNCH_CHECK(ctx);
-            k_gather_product<BS><<<hemo_grid(L.nnz_c, 256), 256, 0, st>>>(L.nnz_c, L.c_seg_ptr, L.c_seg_src, L.r_val,
-                                                                           L.ap_val, C.val);
-            HEMO_LAUNCH_CHECK(ctx);
-        } else {
-            k_numeric_ap<BS><<<hemo_grid((int64_t)A.n * 8, 256), 256, 0, st>>>(A.n, A.rowptr, A.col, A.val, L.p_rowptr, L.p_col,
-                                                                              L.p_val, L.ap_rowptr, L.ap_col, L.ap_val);
-            HEMO_LAUNCH_CHECK(ctx);
-            k_numeric_rap<BS><<<hemo_grid((int64_t)C.n * 32, 256), 256, 0, st>>>(C.n, L.r_rowptr, L.r_col, L.r_val, L.ap_rowptr,
-                                                                                L.ap_col, L.ap_val, L.c_rowptr, L.c_col, C.val);
-            HEMO_LAUNCH_CHECK(ctx);
-        }
+        k_gather_product<BS><<<hemo_grid(L.nnz_ap, 256), 256, 0, st>>>(L.nnz_ap, L.ap_seg_ptr, L.ap_seg_src, L.p_val, A.val,
+                                                                        L.ap_val);
+        HEMO_LAUNCH_CHECK(ctx);
+        k_gather_product<BS><<<hemo_grid(L.nnz_c, 256), 256, 0, st>>>(L.nnz_c, L.c_seg_ptr, L.c_seg_src, L.r_val, L.ap_val,
+                                                                       C.val);
+        HEMO_LAUNCH_CHECK(ctx);
         if (l == 0) HEMO_PROF_END(ctx, HEMO_PROF_RAP);
         HEMO_FILL_SELL(C);
     }
@@ -1578,50 +1354,10 @@ static int vcycle_t(hemo_ctx* ctx, HemoAmg* amg, int l, const areal* b, areal* x
     const int degree = ctx->opts.cheb_degree > 0 ? ctx->opts.cheb_degree : 2;
     const int degree_pre = ctx->opts.cheb_degree_pre > 0 ? ctx->opts.cheb_degree_pre : degree;
     const double ratio = ctx->opts.cheb_ratio > 1.0 ? ctx->opts.cheb_ratio : 4.0;
-    if (l == amg->fuse_level_grid && amg->grid_blocks > 0) {
-        // every remaining level inside one persistent cooperative kernel
-        const HemoCoarseLevel* desc = amg->fuse_desc + (l - amg->fuse_base);
-        int nl = amg->nlev - l, xz = x_is_zero ? 1 : 0, dp = degree_pre, dg = degree, dn = amg->dense_n;
-        double rt = ratio;
-        const double* dinv = amg->dense_inv;
-        void* args[] = {(void*)&desc, (void*)&nl, (void*)&b, (void*)&x, (void*)&xz, (void*)&dp, (void*)&dg, (void*)&rt,
-                        (void*)&dinv, (void*)&dn};
-        const void* fn = (BS == 2) ? (const void*)k_coarse_vcycle_grid<2> : (const void*)k_coarse_vcycle_grid<1>;
-        cudaError_t e = cudaLaunchCooperativeKernel(fn, dim3(amg->grid_blocks), dim3(512), args, 0, st);
-        if (e == cudaSuccess) {
-            ctx->launches++;
-            return 0;
-        }
-        cudaGetLastError();
-        // not available here (or not capturable): per-level kernels + the one-CTA tail from now on
-        ctx->amg[0].grid_blocks = ctx->amg[1].grid_blocks = 0;
-        if (ctx->capturing) HEMO_FAIL(ctx, HEMO_ERETRY, "cooperative launch not capturable: capture is repeated without it");
-    }
-    if (l == amg->fuse_level_cluster && amg->cluster_ctas > 0) {
-        // every remaining level inside one thread-block cluster
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(amg->cluster_ctas); cfg.blockDim = dim3(1024); cfg.stream = st;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = amg->cluster_ctas; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        const HemoCoarseLevel* desc = amg->fuse_desc + (l - amg->fuse_base);
-        const double* dinv = amg->dense_inv;
-        HEMO_CHECK_CUDA(ctx, cudaLaunchKernelEx(&cfg, k_coarse_vcycle_cluster<BS>, desc, amg->nlev - l, b, x, x_is_zero ? 1 : 0,
-                                                degree_pre, degree, ratio, dinv, amg->dense_n));
-        ctx->launches++;
-        return 0;
-    }
     if (l == amg->fuse_level) {
         // every remaining level fits one CTA
-        HEMO_LAUNCH(ctx, k_coarse_vcycle<BS>, 1, 1024, 0, st, amg->fuse_desc + (l - amg->fuse_base), amg->nlev - l, b, x,
-                    x_is_zero ? 1 : 0, degree_pre, degree, ratio, amg->dense_inv, amg->dense_n);
-        return 0;
-    }
-    if (l == amg->nlev - 1) {
-        const int N = amg->dense_n;
-        // exact solve: any previous iterate is simply replaced
-        HEMO_LAUNCH(ctx, k_dense_gemv, hemo_grid((int64_t)N * 32, 256), 256, 0, st, N, amg->dense_inv, b, x);
+        HEMO_LAUNCH(ctx, k_coarse_vcycle<BS>, 1, 1024, 0, st, amg->fuse_desc, amg->nlev - l, b, x, x_is_zero ? 1 : 0, degree, ratio,
+                    amg->dense_inv, amg->dense_n);
         return 0;
     }
     int rc;
@@ -1674,9 +1410,9 @@ int hemo_amg_vcycle(hemo_ctx* ctx, HemoAmg* amg, const double* b, double* x, int
     HemoAmgOp& top = amg->op[0];
     const int64_t N = (int64_t)top.n * amg->bs;
     const int nc = ncycles > 0 ? ncycles : 1;
-    // the top level runs per-level kernels (not inside a fused kernel, not the dense coarsest solve): its first kernel
-    // reads the fp64 right-hand side and its last one writes the fp64 result — no conversion kernels
-    const bool per_level_top = amg->nlev > 1 && amg->fuse_level != 0 && !(amg->fuse_level_grid == 0 && amg->grid_blocks > 0);
+    // the top level runs per-level kernels (it is not inside the fused kernel): its first kernel reads the fp64
+    // right-hand side and its last one writes the fp64 result — no conversion kernels
+    const bool per_level_top = amg->fuse_level > 0;
     if (!per_level_top) HEMO_LAUNCH(ctx, k_to_areal, hemo_grid(N, 256), 256, 0, ctx->stream, N, b, top.b);
     bool wrote64 = false;
     for (int c = 0; c < nc; ++c) {

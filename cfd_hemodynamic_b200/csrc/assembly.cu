@@ -706,51 +706,6 @@ __global__ void k_cell_laplace(int E, const int32_t* __restrict__ cells, const d
     }
 }
 
-// pressure-space convection matrix N_p[a][b] = int phi_a (u_m . grad phi_b) dx, u_m = (u + u_n)/2
-// (the convective part of the pressure convection-diffusion operator F_p of the Schur approximation)
-__global__ void k_cell_pconv(int E, const int32_t* __restrict__ cells, const double* __restrict__ x,
-                             const double* __restrict__ sol, const double* __restrict__ un,
-                             double* __restrict__ Ke /*[9][E]*/) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= E) return;
-    double X[3][2], M[3][2];
-    for (int a = 0; a < 3; ++a) {
-        const int v = cells[3 * (int64_t)c + a];
-        X[a][0] = x[2 * (int64_t)v]; X[a][1] = x[2 * (int64_t)v + 1];
-        M[a][0] = 0.5 * (sol[2 * (int64_t)v] + un[2 * (int64_t)v]);
-        M[a][1] = 0.5 * (sol[2 * (int64_t)v + 1] + un[2 * (int64_t)v + 1]);
-    }
-    const double j00 = X[1][0] - X[0][0], j01 = X[2][0] - X[0][0];
-    const double j10 = X[1][1] - X[0][1], j11 = X[2][1] - X[0][1];
-    const double det = j00 * j11 - j01 * j10;
-    const double i00 = j11 / det, i01 = -j01 / det, i10 = -j10 / det, i11 = j00 / det;
-    double g[3][2];
-    g[1][0] = i00; g[1][1] = i01; g[2][0] = i10; g[2][1] = i11;
-    g[0][0] = -(i00 + i10); g[0][1] = -(i01 + i11);
-    const double dj = fabs(det) / 24.0;
-    for (int b = 0; b < 3; ++b) {
-        double s[3];
-        for (int cc = 0; cc < 3; ++cc) s[cc] = M[cc][0] * g[b][0] + M[cc][1] * g[b][1];
-        const double tot = s[0] + s[1] + s[2];
-        for (int a = 0; a < 3; ++a) Ke[(int64_t)(a * 3 + b) * E + c] = dj * (tot + s[a]);   // sum_c (1 + d_ac) s_c
-    }
-}
-
-__global__ void k_gather_scalar_matrix_areal(int nv2, int64_t nnz_node, int64_t E, const int32_t* __restrict__ seg_ptr,
-                                             const int32_t* __restrict__ seg_src, const double* __restrict__ Ke,
-                                             areal* __restrict__ vals) {
-    const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= nnz_node) return;
-    double acc = 0.0;
-    for (int t = seg_ptr[s]; t < seg_ptr[s + 1]; ++t) {
-        const int src = seg_src[t];
-        const int64_t c = src / nv2;
-        const int ab = src - (int)c * nv2;
-        acc += Ke[(int64_t)ab * E + c];
-    }
-    vals[s] = (areal)acc;
-}
-
 __global__ void k_gather_scalar_matrix(int nv2, int64_t nnz_node, int64_t E, const int32_t* __restrict__ seg_ptr,
                                        const int32_t* __restrict__ seg_src, const double* __restrict__ Ke,
                                        double* __restrict__ vals) {
@@ -1388,58 +1343,6 @@ extern "C" int hemo_assemble_laplace_mass(hemo_ctx* ctx, double* lap_vals_dev, d
     return 0;
 }
 
-// variable-coefficient pressure Laplacian K_kappa with kappa = 1 / (2 rho (1/dt + c_u |u_m| / h)) per cell:
-// the inertial part of  1/2 B A00^-1 B^T  (mass + convection on the diagonal of A00)
-__global__ void k_cell_kappa_laplace(int E, const int32_t* __restrict__ cells, const double* __restrict__ x,
-                                     const double* __restrict__ h, const double* __restrict__ sol,
-                                     const double* __restrict__ un, double rho, double dt, double c_u,
-                                     double* __restrict__ Ke /*[9][E]*/) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= E) return;
-    double X[3][2], um[2] = {0.0, 0.0};
-    for (int a = 0; a < 3; ++a) {
-        const int v = cells[3 * (int64_t)c + a];
-        X[a][0] = x[2 * (int64_t)v]; X[a][1] = x[2 * (int64_t)v + 1];
-        um[0] += 0.5 * (sol[2 * (int64_t)v] + un[2 * (int64_t)v]) / 3.0;
-        um[1] += 0.5 * (sol[2 * (int64_t)v + 1] + un[2 * (int64_t)v + 1]) / 3.0;
-    }
-    const double j00 = X[1][0] - X[0][0], j01 = X[2][0] - X[0][0];
-    const double j10 = X[1][1] - X[0][1], j11 = X[2][1] - X[0][1];
-    const double det = j00 * j11 - j01 * j10;
-    const double i00 = j11 / det, i01 = -j01 / det, i10 = -j10 / det, i11 = j00 / det;
-    double g[3][2];
-    g[1][0] = i00; g[1][1] = i01; g[2][0] = i10; g[2][1] = i11;
-    g[0][0] = -(i00 + i10); g[0][1] = -(i01 + i11);
-    const double speed = sqrt(um[0] * um[0] + um[1] * um[1]);
-    const double kappa = 1.0 / (2.0 * rho * (1.0 / dt + c_u * speed / h[c]));
-    const double sc = kappa * 0.5 * fabs(det);
-    for (int a = 0; a < 3; ++a)
-        for (int b = 0; b < 3; ++b) Ke[(int64_t)(a * 3 + b) * E + c] = sc * (g[a][0] * g[b][0] + g[a][1] * g[b][1]);
-}
-
-// S_hat = A11 (PSPG block of the Jacobian) + K_kappa, identity on masked / Dirichlet pressure nodes
-__global__ void k_build_schur_operator(int n, int64_t nnz_node, const int32_t* __restrict__ nrowptr,
-                                       const int32_t* __restrict__ rowof, const int32_t* __restrict__ ncol,
-                                       const double* __restrict__ vals, const double* __restrict__ klap,
-                                       const uint8_t* __restrict__ dofflag, const uint8_t* __restrict__ mask,
-                                       areal* __restrict__ out) {
-    const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= nnz_node) return;
-    const int i = rowof[s], j = ncol[s];
-    const bool fi = (dofflag && dofflag[2 * (int64_t)n + i]) || (mask && mask[i]);
-    const bool fj = (dofflag && dofflag[2 * (int64_t)n + j]) || (mask && mask[j]);
-    double v;
-    if (fi || fj) {
-        v = (i == j) ? 1.0 : 0.0;
-    } else {
-        const int r0 = nrowptr[i];
-        const int deg = nrowptr[i + 1] - r0;
-        const int t = (int)(s - r0);
-        v = vals[6 * nnz_node + 3 * (int64_t)r0 + 2 * deg + t] + klap[s];
-    }
-    out[s] = (areal)v;
-}
-
 // SELFP: Sp = A11 - A10 diag(A00)^-1 A01 on the distance-2 node graph, straight from the
 // monolithic Jacobian values (PETSc MatSchurComplementGetPmat with SELFP, reference
 // src/solvers/stabilized_schur.py:235).  One thread per Sp entry.
@@ -1498,56 +1401,4 @@ extern "C" int hemo_pc_set_schur_selfp(hemo_ctx* ctx, const double* vals_dev, do
                                                                    amg.op[0].val);
     HEMO_LAUNCH_CHECK(ctx);
     return hemo_amg_numeric_shift(ctx, &amg, coarse_shift);
-}
-
-extern "C" int hemo_set_schur_mask(hemo_ctx* ctx, const uint8_t* node_mask_dev) {
-    if (!ctx) return HEMO_EINVAL;
-    if (!ctx->cells) HEMO_FAIL(ctx, HEMO_ESTATE, "hemo_set_mesh must precede hemo_set_schur_mask");
-    if (!node_mask_dev) { cudaFree(ctx->schur_mask); ctx->schur_mask = nullptr; return 0; }
-    return hemo_upload(ctx, &ctx->schur_mask, node_mask_dev, (size_t)ctx->n, true);
-}
-
-extern "C" int hemo_pc_set_schur_operator(hemo_ctx* ctx, const double* x_dev, const double* un_dev,
-                                          const double* vals_dev, double c_u, double coarse_shift) {
-    if (!ctx || !x_dev || !un_dev || !vals_dev) return HEMO_EINVAL;
-    if (!ctx->cells || !ctx->nrowptr || !ctx->have_par) HEMO_FAIL(ctx, HEMO_ESTATE, "mesh / node graph / params not set");
-    if (!ctx->amg[1].ready) HEMO_FAIL(ctx, HEMO_ESTATE, "pressure AMG hierarchy not finalized");
-    if (ctx->nv != 3 || ctx->dim != 2) HEMO_FAIL(ctx, HEMO_ESTATE, "the assembled Schur operator is implemented for triangles only");
-    const int E = ctx->E, n = ctx->n;
-    int rc;
-    if ((rc = ensure_elem(ctx, (size_t)9 * E, 0))) return rc;
-    if (!ctx->schur_tmp && (rc = hemo_alloc(ctx, &ctx->schur_tmp, (size_t)ctx->nnz_node))) return rc;
-    cudaStream_t st = ctx->stream;
-    k_cell_kappa_laplace<<<hemo_grid(E, 256), 256, 0, st>>>(E, ctx->cells, ctx->x, ctx->h, x_dev, un_dev, ctx->par.rho,
-                                                           ctx->par.dt, c_u, ctx->Ae);
-    HEMO_LAUNCH_CHECK(ctx);
-    k_gather_scalar_matrix<<<hemo_grid(ctx->nnz_node, 256), 256, 0, st>>>(9, ctx->nnz_node, E, ctx->mseg_ptr, ctx->mseg_src,
-                                                                          ctx->Ae, ctx->schur_tmp);
-    HEMO_LAUNCH_CHECK(ctx);
-    k_build_schur_operator<<<hemo_grid(ctx->nnz_node, 256), 256, 0, st>>>(
-        n, ctx->nnz_node, ctx->nrowptr, ctx->rowof, ctx->ncol, vals_dev, ctx->schur_tmp,
-        ctx->have_bc ? ctx->dofflag : nullptr, ctx->schur_mask, ctx->amg[1].op[0].val);
-    HEMO_LAUNCH_CHECK(ctx);
-    return hemo_amg_numeric_shift(ctx, &ctx->amg[1], coarse_shift);
-}
-
-extern "C" int hemo_pc_set_convection(hemo_ctx* ctx, const double* x_dev, const double* un_dev, double coef) {
-    if (!ctx) return HEMO_EINVAL;
-    ctx->npconv_coef = coef;
-    if (coef == 0.0) return 0;
-    HEMO_2D_ONLY(ctx, "the pressure convection term");
-    if (!x_dev || !un_dev) return HEMO_EINVAL;
-    if (!ctx->cells || !ctx->nrowptr) HEMO_FAIL(ctx, HEMO_ESTATE, "mesh / node graph not set");
-    if (ctx->nv != 3) HEMO_FAIL(ctx, HEMO_ESTATE, "the pressure convection term is implemented for triangles only");
-    const int E = ctx->E;
-    int rc;
-    if ((rc = ensure_elem(ctx, (size_t)9 * E, 0))) return rc;
-    if (!ctx->npconv && (rc = hemo_alloc(ctx, &ctx->npconv, (size_t)ctx->nnz_node))) return rc;
-    cudaStream_t st = ctx->stream;
-    k_cell_pconv<<<hemo_grid(E, 256), 256, 0, st>>>(E, ctx->cells, ctx->x, x_dev, un_dev, ctx->Ae);
-    HEMO_LAUNCH_CHECK(ctx);
-    k_gather_scalar_matrix_areal<<<hemo_grid(ctx->nnz_node, 256), 256, 0, st>>>(9, ctx->nnz_node, E, ctx->mseg_ptr,
-                                                                                ctx->mseg_src, ctx->Ae, ctx->npconv);
-    HEMO_LAUNCH_CHECK(ctx);
-    return 0;
 }

@@ -30,8 +30,6 @@ typedef float2 areal2;
 typedef float4 areal4;
 #endif
 
-#define HEMO_ERETRY (-3)      // internal: a stream capture has to be repeated (never returned through the C ABI)
-
 struct HemoRule {
     int nq;
     int alias;                // lowest block id with an identical rule
@@ -73,7 +71,7 @@ struct HemoAmgLevel {
     int32_t *ap_rowptr = nullptr, *ap_col = nullptr; areal* ap_val = nullptr;
     int32_t *c_rowptr = nullptr, *c_col = nullptr;
     int64_t nnz_p = 0, nnz_ap = 0, nnz_c = 0;
-    // precomputed gather lists of the numeric Galerkin product (hierarchy 0 only):
+    // precomputed gather lists of the numeric Galerkin product:
     // AP[s] = sum_k p_val[src.x] * A[src.y],  C[s] = sum_k r_val[src.x] * AP[src.y]
     int32_t* ap_seg_ptr = nullptr; int2* ap_seg_src = nullptr;
     int32_t* c_seg_ptr = nullptr;  int2* c_seg_src = nullptr;
@@ -90,19 +88,7 @@ struct HemoCoarseLevel {
     const double* lmax;
 };
 
-#define HEMO_FUSE_MAX_NODES 256    // levels at or below this size run inside one CTA (HEMO_FUSE_MAX=<nodes> overrides)
-#define HEMO_FUSE_STRONG_PRE_NODES 256   // levels at or below this size pre-smooth with the full Chebyshev degree
-// Levels (below the finest) at or below this size run inside the cooperative persistent-grid kernel.  0 = off, the
-// default: measured on a B200 (lid cavity 707^2) the grid.sync between the ~40 phases costs more than the graph-
-// scheduled per-level launches it replaces (36.9 vs 29.7 ms per time step); HEMO_GRID_FUSE_MAX=<nodes> turns it on.
-#define HEMO_GRID_FUSE_MAX_NODES 0
-// Levels at or below this size (and above HEMO_FUSE_MAX_NODES) run inside ONE thread-block cluster, phases separated
-// by the hardware cluster barrier (~0.2 us against 3-5 us for a grid-wide barrier or a kernel boundary).  0 = off, the
-// default: measured on a B200 (lid cavity 707^2, levels of 9.6 k / 1.2 k nodes) 16 SMs do not hide the three dependent
-// L2 accesses of a phase as well as 150-CTA launches spread over the GPU do (29.5 ms per time step with a cluster of
-// 16, 32.6 with 8, against 27.6 with per-level launches).  HEMO_CLUSTER_FUSE_MAX=<nodes> turns it on,
-// HEMO_CLUSTER_CTAS=<2..16> sets the cluster size.
-#define HEMO_CLUSTER_FUSE_MAX_NODES 0
+#define HEMO_FUSE_MAX_NODES 256    // levels at or below this size run inside one CTA (k_coarse_vcycle)
 
 struct HemoAmg {
     // cached CUDA graph of hemo_amg_apply(b, x, ncycles) (replicated global pressure solve)
@@ -115,12 +101,7 @@ struct HemoAmg {
     // optional level-0 pattern that differs from the mesh node graph (SELFP: distance-2 graph)
     int32_t *fine_rowptr = nullptr, *fine_col = nullptr, *fine_rowof = nullptr;
     int64_t fine_nnz = 0;
-    int fuse_level = -1;           // first level handled by the one-CTA fused kernel (-1: none)
-    int fuse_level_grid = -1;      // first level handled by the cooperative persistent-grid kernel (-1: none)
-    int fuse_base = -1;            // level of fuse_desc[0]
-    int grid_blocks = 0;           // CTAs of the cooperative kernel (one per SM); 0: cooperative launch unavailable
-    int fuse_level_cluster = -1;   // first level handled by the one-cluster fused kernel (-1: none)
-    int cluster_ctas = 0;          // CTAs of that cluster; 0: cluster launch unavailable
+    int fuse_level = -1;           // first level handled by the one-CTA fused kernel (-1: not finalized)
     HemoCoarseLevel* fuse_desc = nullptr;   // device array, one per level from fuse_level
     double* lmax_dev = nullptr;    // HEMO_MAX_LEVELS Gershgorin bounds kept on the device
     int bs = 1;
@@ -242,10 +223,6 @@ struct hemo_ctx {
     double schur_mass_coef = 0.0, schur_lap_coef = 0.0;
     HemoAmg amg[2];
     const double* mass = nullptr;   // lumped pressure mass (borrowed, n)
-    uint8_t* schur_mask = nullptr;  // n: identity rows/cols of the assembled Schur operator (open / ghost nodes)
-    double* schur_tmp = nullptr;    // nnz_node scratch
-    areal* npconv = nullptr;        // nnz_node: pressure-space convection matrix N_p (PCD term of the Schur approx.)
-    double npconv_coef = 0.0;       // 0: term disabled
     areal2* a01 = nullptr;          // nnz_node: compact copy of the A01 block (u rows x p cols) for the PC
     uint8_t* pc_mask = nullptr;     // n: nodes excluded from the local preconditioner (ghosts)
     double* kry_coef = nullptr;     // device scratch for hemo_vec_maxpy coefficients (512)

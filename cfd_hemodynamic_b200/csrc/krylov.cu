@@ -595,7 +595,6 @@ static int fg_iteration(hemo_ctx* ctx, const double* vals_dev) {
     if (rc != 0 || e != cudaSuccess || !g) {
         cudaGetLastError();
         if (g) cudaGraphDestroy(g);
-        if (rc == HEMO_ERETRY) return fg_iteration(ctx, vals_dev);     // captured again without the cooperative kernel
         if (rc) return rc;
         ctx->use_graph = 0;
         return fg_iteration_body(ctx, vals_dev);

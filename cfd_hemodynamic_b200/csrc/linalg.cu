@@ -68,9 +68,8 @@ void hemo_drop_solver_state(hemo_ctx* ctx) {
     ctx->kry_restart = 0;
     hemo_krylov_invalidate(ctx);
     ctx->kry.m = 0; ctx->kry.last_its = 0;
-    cudaFree(ctx->pc_mask); cudaFree(ctx->schur_mask); cudaFree(ctx->schur_tmp); cudaFree(ctx->npconv);
-    ctx->pc_mask = ctx->schur_mask = nullptr; ctx->schur_tmp = nullptr; ctx->npconv = nullptr;
-    ctx->npconv_coef = 0.0;
+    cudaFree(ctx->pc_mask);
+    ctx->pc_mask = nullptr;
     ctx->mass = nullptr;
     ctx->amg[0].ready = ctx->amg[1].ready = false;
 }

@@ -173,34 +173,15 @@ k_a01_residual_row(int n, const int32_t* __restrict__ nrowptr, const int32_t* __
     tu[2 * (int64_t)i + 1] = ru[2 * (int64_t)i + 1] - a1;
 }
 
-// c = N_p q on the node graph (4 lanes per row)
-__global__ void __launch_bounds__(256)
-k_node_spmv_scalar(int n, const int32_t* __restrict__ nrowptr, const int32_t* __restrict__ ncol,
-                   const areal* __restrict__ val, const double* __restrict__ q, double* __restrict__ out) {
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = gt >> 2, lane = gt & 3;
-    const bool ok = i < n;
-    const int r0 = ok ? nrowptr[i] : 0, r1 = ok ? nrowptr[i + 1] : 0;
-    hemo_pdl_wait();
-    hemo_pdl_trigger();
-    double a = 0.0;
-    for (int s = r0 + lane; s < r1; s += 4) a = fma((double)val[s], q[ncol[s]], a);
-    a += __shfl_down_sync(0xffffffffu, a, 2, 4);
-    a += __shfl_down_sync(0xffffffffu, a, 1, 4);
-    if (ok && lane == 0) out[i] = a;
-}
-
-// z_p = (c_m t_p + c_c (N_p q)) / mass + c_L q_p ; Dirichlet pressure dofs: z_p = r_p
-__global__ void k_schur_combine(int n, double cm, double cl, double cc, const double* __restrict__ tp,
-                                const double* __restrict__ mass, const double* __restrict__ qp,
-                                const double* __restrict__ conv, const uint8_t* __restrict__ dofflag /* pressure part, n */,
+// z_p = c_m t_p / mass + c_L q_p ; Dirichlet pressure dofs: z_p = r_p
+__global__ void k_schur_combine(int n, double cm, double cl, const double* __restrict__ tp, const double* __restrict__ mass,
+                                const double* __restrict__ qp, const uint8_t* __restrict__ dofflag /* pressure part, n */,
                                 const double* __restrict__ rp, double* __restrict__ zp) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     hemo_pdl_wait();
     hemo_pdl_trigger();
     if (i >= n) return;
     double v = cm * tp[i] / mass[i] + cl * qp[i];
-    if (conv) v += cc * conv[i] / mass[i];
     if (dofflag && dofflag[i]) v = rp[i];
     zp[i] = v;
 }
@@ -492,7 +473,7 @@ extern "C" int hemo_amg_apply(hemo_ctx* ctx, int which, const double* b_dev, dou
     if (rc != 0 || e != cudaSuccess || !g) {
         cudaGetLastError();
         if (g) cudaGraphDestroy(g);
-        if (rc && rc != HEMO_ERETRY) return rc;
+        if (rc) return rc;
         return hemo_amg_vcycle(ctx, &amg, b_dev, x_dev, ncycles);
     }
     if (amg.apply_exec) { cudaGraphExecDestroy(amg.apply_exec); amg.apply_exec = nullptr; }
@@ -520,17 +501,10 @@ extern "C" int hemo_amg_level_info(hemo_ctx* ctx, int which, int level, int64_t*
     const HemoAmg& amg = ctx->amg[which];
     if (!amg.ready || level < 0 || level >= amg.nlev) return HEMO_EINVAL;
     const HemoAmgOp& o = amg.op[level];
-    // the order of the tests follows vcycle_t: a level runs in the first fused kernel whose range covers it; the grid
-    // kernel counts only while its cooperative launch is available (grid_blocks drops to 0 when it fails)
-    int scope = HEMO_AMG_SCOPE_LEVEL;
-    if (amg.grid_blocks > 0 && amg.fuse_level_grid >= 0 && level >= amg.fuse_level_grid) scope = HEMO_AMG_SCOPE_GRID;
-    else if (amg.cluster_ctas > 0 && amg.fuse_level_cluster >= 0 && level >= amg.fuse_level_cluster) scope = HEMO_AMG_SCOPE_CLUSTER;
-    else if (amg.fuse_level >= 0 && level >= amg.fuse_level) scope = HEMO_AMG_SCOPE_CTA;
-    else if (level == amg.nlev - 1) scope = HEMO_AMG_SCOPE_DENSE;
     out[0] = o.n;
     out[1] = o.nnzb;
     out[2] = o.sell_ptr ? o.sell_entries : 0;
-    out[3] = scope;
+    out[3] = level >= amg.fuse_level ? HEMO_AMG_SCOPE_CTA : HEMO_AMG_SCOPE_LEVEL;
     return 0;
 }
 
@@ -560,14 +534,8 @@ int hemo_pc_apply_body(hemo_ctx* ctx, const double* vals_dev, const double* r_de
         if ((rc = coarse_pressure_join(ctx, qp))) return rc;
         HEMO_PROF_END(ctx, HEMO_PROF_COARSE);
     }
-    const bool pcd = ctx->npconv_coef != 0.0 && ctx->npconv;
-    if (pcd) {
-        // pressure convection-diffusion term: S^-1 ~ 2 Mp^-1 Fp Lp^-1 with Fp = rho/dt Mp + rho/2 Np + mu/2 Lp
-        HEMO_LAUNCH(ctx, k_node_spmv_scalar, hemo_grid((int64_t)n * 4, 256), 256, 0, st, n, ctx->nrowptr, ctx->ncol, ctx->npconv,
-                    qp, ctx->pc_tmp_u2);
-    }
-    HEMO_LAUNCH(ctx, k_schur_combine, hemo_grid(n, 256), 256, 0, st, n, ctx->opts.schur_mass_coef, ctx->opts.schur_lap_coef,
-                ctx->npconv_coef, tp, ctx->mass, qp, pcd ? ctx->pc_tmp_u2 : nullptr, pressure_flags(ctx), rp, zp);
+    HEMO_LAUNCH(ctx, k_schur_combine, hemo_grid(n, 256), 256, 0, st, n, ctx->opts.schur_mass_coef, ctx->opts.schur_lap_coef, tp,
+                ctx->mass, qp, pressure_flags(ctx), rp, zp);
     if (ctx->opts.project_pressure && (rc = hemo_remove_mean(ctx, n, zp))) return rc;
     }   // else: z_p was provided by the caller (global pressure solve of the multi-GPU driver)
     if (ctx->dim == 3)    // t_u = r_u - A01 z_p, then damped block-Jacobi sweeps on A00 (amg_cycles_u * 4 sweeps)
@@ -610,7 +578,6 @@ static int pc_build_graph(hemo_ctx* ctx, const double* vals_dev) {
     if (rc != 0 || e != cudaSuccess || !g) {
         cudaGetLastError();
         if (g) cudaGraphDestroy(g);
-        if (rc == HEMO_ERETRY) return pc_build_graph(ctx, vals_dev);
         ctx->use_graph = 0;
         if (rc) return rc;
         return 0;
@@ -690,7 +657,6 @@ extern "C" int hemo_ctx_destroy(hemo_ctx* ctx) {
     hemo_amg_free(&ctx->amg[0]); hemo_amg_free(&ctx->amg[1]);
     if (ctx->pc_graph_exec) cudaGraphExecDestroy(ctx->pc_graph_exec);
     if (ctx->pc_graph) cudaGraphDestroy(ctx->pc_graph);
-    cudaFree(ctx->npconv); cudaFree(ctx->schur_mask); cudaFree(ctx->schur_tmp);
     cudaFree(ctx->wss_cell2t); cudaFree(ctx->wss_tmp);
     free(ctx->qrules);
     free(ctx->p2rules);

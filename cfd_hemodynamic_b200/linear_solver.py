@@ -22,18 +22,18 @@ class BlockSchurSolver:
                  amg_cycles_u: int = 1, amg_cycles_p: int = 1, cheb_degree: int = 2, cheb_ratio: float = 4.0, cheb_degree_pre: int = 1,
                  project_pressure: bool = False, smooth_prolongator: bool = True, strength_theta: float = 0.08,
                  schur_mass_coef: float | None = None, schur_lap_coef: float | None = None,
-                 schur_mode: str = "laplace", schur_cu: float = 1.0):
+                 schur_mode: str = "laplace"):
+        # "laplace": S^-1 ~ mu Mp^-1 + (2 rho/dt) Lp^-1 (Cahouet–Chabard, constant operators);
+        # "selfp": S^-1 ~ Sp^-1 with the reference's Sp = A11 - A10 diag(A00)^-1 A01, re-formed by every setup()
+        if schur_mode not in ("laplace", "selfp"):
+            raise ValueError(f"schur_mode {schur_mode!r}: 'laplace' and 'selfp' are implemented")
         self.hemo = hemo
         n = nrowptr.shape[0] - 1
         self.n = n
-        # "laplace": S^-1 ~ mu Mp^-1 + (2 rho/dt) Lp^-1 (Cahouet–Chabard, constant operators);
-        # "assembled": S^-1 ~ mu Mp^-1 + (A11 + K_kappa)^-1 re-formed for every new Jacobian
         self.schur_mode = schur_mode
-        self.schur_cu = float(schur_cu)
-        if schur_mode in ("assembled", "selfp") and schur_lap_coef is None:
-            schur_lap_coef = 1.0
-        if schur_mode == "selfp" and schur_mass_coef is None:
-            schur_mass_coef = 0.0
+        if schur_mode == "selfp":
+            schur_lap_coef = 1.0 if schur_lap_coef is None else schur_lap_coef
+            schur_mass_coef = 0.0 if schur_mass_coef is None else schur_mass_coef
         # a pressure operator without any Dirichlet row is singular on the coarsest level
         no_pin = len(p_dirichlet_nodes) == 0 and (schur_mode == "selfp" or p_open_nodes is None or len(p_open_nodes) == 0)
         self.coarse_shift = 1e-8 if (project_pressure or no_pin) else 0.0
@@ -65,7 +65,6 @@ class BlockSchurSolver:
             self.lap = hemo.torch.from_numpy(np.ascontiguousarray(lap_host)).to(hemo.device)
             L = sp.csr_matrix((lap_host, ncol, nrowptr), shape=(n, n))
             pmask |= omask
-            hemo.set_schur_mask(hemo.torch.from_numpy(omask.astype(np.uint8)).to(hemo.device))
         self.levels = []
         fine_p = None
         if schur_mode == "selfp":
@@ -77,12 +76,9 @@ class BlockSchurSolver:
             # SELFP carries the boundary conditions algebraically: only true Dirichlet pressure dofs are fixed
             pmask = np.zeros(n, dtype=bool)
             pmask[np.asarray(p_dirichlet_nodes, dtype=np.int64)] = True
-            hemo.set_schur_mask(None)
         # tetrahedra: the velocity block is handled by block-Jacobi sweeps inside the library
         # (no 3x3-block hierarchy yet, DESIGN.md §5b); only the scalar pressure hierarchy is built
         tet = getattr(hemo, "dim", 2) == 3
-        if tet and schur_mode not in ("laplace", "selfp"):
-            raise ValueError("tetrahedra: schur_mode 'laplace' and 'selfp' are implemented")
         for which, mask, max_coarse in ((0, umask, 80), (1, pmask, 160)):
             if tet and which == 0:
                 self.levels.append([])
@@ -102,15 +98,10 @@ class BlockSchurSolver:
             self.opts["max_it"] = max_it
         self.hemo.set_solver_opts(**self.opts)
 
-    def setup(self, vals, x=None, un=None):
+    def setup(self, vals):
         """pc.setUp() for a new Jacobian."""
         if self.schur_mode == "selfp":
             self.hemo.pc_set_schur_selfp(vals, self.coarse_shift)
-            self.hemo.pc_setup(vals, None, self.mass if self._first else None)
-            self._first = False
-            return
-        if self.schur_mode == "assembled":
-            self.hemo.pc_set_schur_operator(x, un, vals, self.schur_cu, self.coarse_shift)
             self.hemo.pc_setup(vals, None, self.mass if self._first else None)
             self._first = False
             return

@@ -81,15 +81,12 @@ class StabilizedSchurB200(SolverBase):
         # "newton": PCSetUp for every Jacobian like the reference (SNES lag 1);
         # "step": once per time step, later Newton iterations reuse the hierarchy
         self.pc_rebuild = str(kw.pop("pc_rebuild", "step"))
-        # coefficient of the pressure convection-diffusion term of the Schur approximation in
-        # units of rho (1: S^-1 ~ 2 Mp^-1 Fp Lp^-1 with the convective part of Fp; 0: Cahouet-Chabard)
-        self.schur_convection = float(kw.pop("schur_convection", 0.0))
         # treatment of open (traction) boundary nodes in the pressure operator of the Schur
         # approximation: "dirichlet" (identity rows) or "natural" (regular rows)
         self.schur_open = str(kw.pop("schur_open", "dirichlet"))
         self._pc_kw = {k: kw.pop(k) for k in list(kw) if k in (
             "amg_cycles_u", "amg_cycles_p", "cheb_degree", "cheb_ratio", "cheb_degree_pre", "smooth_prolongator",
-            "strength_theta", "schur_mass_coef", "schur_lap_coef", "schur_mode", "schur_cu")}
+            "strength_theta", "schur_mass_coef", "schur_lap_coef", "schur_mode")}
         self._rules = kw.pop("quadrature", None)
         self._device_index = int(kw.pop("device", 0))
         # host_only: build spaces / BC tables / facet tables but create no CUDA context
@@ -283,7 +280,7 @@ class StabilizedSchurB200(SolverBase):
             dt=float(self.dt.value), rho=float(self.rho.value), mu=float(self.mu.value),
             restart=self.ksp_restart, max_it=self.ksp_max_it, rtol=self.ksp_rtol, atol=self.ksp_atol,
             project_pressure=self._nullspace, **self._pc_kw)
-        self.linear.setup(self.d_vals, self.d_x, self.d_un)
+        self.linear.setup(self.d_vals)
 
     def _test_nullspace(self) -> bool:
         """nullsp.test(A): is the constant-pressure vector in the kernel of A?
@@ -318,9 +315,7 @@ class StabilizedSchurB200(SolverBase):
         for it in range(self.snes_max_it):
             hemo.assemble_jacobian(x, self.d_un, self.d_vals)
             if it == 0 or self.pc_rebuild == "newton":
-                if self.schur_convection != 0.0:
-                    hemo.pc_set_convection(x, self.d_un, self.schur_convection * float(self.rho.value))
-                self.linear.setup(self.d_vals, x, self.d_un)
+                self.linear.setup(self.d_vals)
             try:
                 kits, _ = self.linear.solve(self.d_vals, f, y)
             except HemoDiverged:

@@ -162,7 +162,7 @@ class StabilizedSchurTetB200(StabilizedSchurB200):
             dt=float(self.dt.value), rho=float(self.rho.value), mu=float(self.mu.value),
             restart=self.ksp_restart, max_it=self.ksp_max_it, rtol=self.ksp_rtol, atol=self.ksp_atol,
             project_pressure=self._nullspace, **self._pc_kw)
-        self.linear.setup(self.d_vals, self.d_x, self.d_un)
+        self.linear.setup(self.d_vals)
 
     def _test_nullspace(self) -> bool:
         if not self._tet:

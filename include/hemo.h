@@ -206,8 +206,7 @@ int hemo_assemble_laplace_mass(hemo_ctx* ctx, double* lap_vals_dev, double* mass
  *   block-Jacobi sweeps).
  *   hemo_pc_set_schur_selfp (SELFP from the 3-D CSR values), hemo_wall_shear_stress (3n output; per-vertex
  *   gather in a fixed order, bitwise reproducible), hemo_early_stop_norms, hemo_l2_norm_sq (bs = 1 or 3).
- * Still 2-D only (HEMO_ESTATE on tetrahedra): hemo_boundary_force, the assembled Schur operator and pressure
- * convection term, partition masks. */
+ * Still 2-D only (HEMO_ESTATE on tetrahedra): hemo_boundary_force, partition masks. */
 int hemo_set_body_force3(hemo_ctx* ctx, const double* f3_host);
 int hemo_tet_set_quadrature(hemo_ctx* ctx, int block, const double* pts_host, const double* wts_host, int nq);
 int hemo_tet_element_tensors(hemo_ctx* ctx, int n_nodes, int n_cells, const double* x_dev,
@@ -281,11 +280,9 @@ int hemo_amg_apply(hemo_ctx* ctx, int which, const double* b_dev, double* x_dev,
 int hemo_amg_get_level_values(hemo_ctx* ctx, int which, int level, double* vals_dev, int64_t capacity);
 /* Which kernels run level `level` of hierarchy `which` (read-only, after hemo_amg_finalize):
  * out[0] = block rows n, out[1] = blocks nnzb, out[2] = entries of the sliced-ELL copy (0: CSR kernels),
- * out[3] = HEMO_AMG_SCOPE_*: the per-level kernels, one of the fused coarse V-cycle kernels (one CTA,
- * cooperative grid, thread-block cluster) or the dense coarsest-level solve.  Read at the time of the
- * call: the grid scope falls back to the others once a cooperative launch has failed. */
-enum { HEMO_AMG_SCOPE_LEVEL = 0, HEMO_AMG_SCOPE_CTA = 1, HEMO_AMG_SCOPE_GRID = 2, HEMO_AMG_SCOPE_CLUSTER = 3,
-       HEMO_AMG_SCOPE_DENSE = 4 };
+ * out[3] = HEMO_AMG_SCOPE_*: the per-level kernels or the fused coarse V-cycle kernel (one CTA, which also
+ * applies the dense inverse of the coarsest level). */
+enum { HEMO_AMG_SCOPE_LEVEL = 0, HEMO_AMG_SCOPE_CTA = 1 };
 int hemo_amg_level_info(hemo_ctx* ctx, int which, int level, int64_t out[4]);
 /* ---- multi-GPU building blocks (domain decomposition, one partition per GPU) ----------
  * The host driver (cfd_hemodynamic_b200/parallel.py) exchanges ghost values and sums the
@@ -353,16 +350,6 @@ int hemo_set_poll_interval(hemo_ctx* ctx, int every);
 /* 1 (default): hemo_pc_setup captures one preconditioner application as a CUDA
  * graph (needs a non-default stream) and hemo_pc_apply replays it; 0: direct launches. */
 int hemo_use_graph(hemo_ctx* ctx, int on);
-/* Assembled Schur operator (alternative to the constant Laplacian): level 0 of the pressure
- * hierarchy becomes  S_hat = A11 + K_kappa  with A11 the PSPG block of the current Jacobian
- * (exact, like SELFP keeps it: src/solvers/stabilized_schur.py:235) and K_kappa a pressure
- * Laplacian with the per-cell coefficient kappa = 1 / (2 rho (1/dt + c_u |u_m| / h)) standing for
- * 1/2 B A00^-1 B^T; the hierarchy is re-formed numerically.  Nodes flagged by
- * hemo_set_schur_mask (open boundaries, ghosts) and Dirichlet pressure dofs get identity rows.
- * Use with schur_lap_coef = 1. */
-int hemo_set_schur_mask(hemo_ctx* ctx, const uint8_t* node_mask_dev);
-int hemo_pc_set_schur_operator(hemo_ctx* ctx, const double* x_dev, const double* un_dev,
-                               const double* vals_dev, double c_u, double coarse_shift);
 /* SELFP Schur preconditioning matrix like the reference's (src/solvers/stabilized_schur.py:235):
  * Sp = A11 - A10 diag(A00)^-1 A01, formed on the device from the monolithic Jacobian on the
  * distance-2 node graph given with hemo_amg_set_fine_pattern(which = 1) (host CSR arrays, before
@@ -370,11 +357,6 @@ int hemo_pc_set_schur_operator(hemo_ctx* ctx, const double* x_dev, const double*
  * Use with schur_mass_coef = 0, schur_lap_coef = 1. */
 int hemo_amg_set_fine_pattern(hemo_ctx* ctx, int which, const int32_t* rowptr_host, const int32_t* col_host);
 int hemo_pc_set_schur_selfp(hemo_ctx* ctx, const double* vals_dev, double coarse_shift);
-/* Optional pressure convection-diffusion term of the Schur approximation: assembles
- * N_p = int phi_a (u_m . grad phi_b) on the pressure space from the current state and adds
- * coef * Mp^-1 N_p Lp^-1 r to S^-1 r (coef = rho for the mid-point scheme; 0 disables).
- * Call before hemo_pc_setup. */
-int hemo_pc_set_convection(hemo_ctx* ctx, const double* x_dev, const double* un_dev, double coef);
 /* z = M^{-1} r (one application of the block preconditioner). */
 int hemo_pc_apply(hemo_ctx* ctx, const double* vals_dev, const double* r_dev, double* z_dev);
 /* KSPSolve: right-preconditioned FGMRES(restart) on J y = b with zero initial

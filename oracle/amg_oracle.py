@@ -20,7 +20,7 @@ import scipy.sparse as sp
 AMG_TOL = 1e-5
 
 # levels handled by a fused coarse V-cycle kernel that have at most this many nodes pre-smooth with the full
-# Chebyshev degree (HEMO_FUSE_STRONG_PRE_NODES in hemo_internal.cuh)
+# Chebyshev degree (HEMO_FUSE_MAX_NODES in hemo_internal.cuh: every level of the one-CTA kernel)
 STRONG_PRE_NODES = 256
 
 

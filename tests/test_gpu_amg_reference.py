@@ -4,9 +4,8 @@ oracle/amg_oracle.py, on every kernel path of amg.cu.
 Each configuration is a fresh library context on a lid-cavity Jacobian (walls and lid: Dirichlet multiplicity 2 at
 the top corners, empty prolongator rows on the boundary).  Which kernels run depends on the level size, the row
 length, the Chebyshev degrees, the cycle count, the prolongator density and the environment variables HEMO_PDL
-(read at context creation), HEMO_NO_GRAPH (read by `Hemo()`), HEMO_SELL, HEMO_FUSE_MAX, HEMO_GRID_FUSE_MAX and
-HEMO_CLUSTER_FUSE_MAX (read by hemo_amg_finalize); every row asserts the path it claims through
-`Hemo.amg_level_info`.
+(read at context creation), HEMO_NO_GRAPH (read by `Hemo()`) and HEMO_SELL (read by hemo_amg_finalize); every row
+asserts the path it claims through `Hemo.amg_level_info`.
 
 The hierarchies are stored and cycled in single precision; the model rounds only the stored operators.  Both
 ||e||_2 / ||x_ref||_2 and max|e| / max|x_ref| must stay below oracle.amg_oracle.AMG_TOL (the max norm catches one
@@ -78,10 +77,10 @@ def _velocity_oracle(c, mask=None):
 
 
 def _paths(c, which):
-    """amg_level_info of every level, and the levels inside a fused coarse V-cycle kernel."""
+    """amg_level_info of every level, and the levels inside the fused coarse V-cycle kernel."""
     h = c["hemo"]
     info = [h.amg_level_info(which, l) for l in range(len(c["s"].levels[which]) + 1)]
-    return info, {l for l, d in enumerate(info) if d["scope"] in ("cta", "grid", "cluster")}
+    return info, {l for l, d in enumerate(info) if d["scope"] == "cta"}
 
 
 def _prolongation_kernel(c, which):
@@ -188,10 +187,6 @@ CASES = [
      dict(degree=3, degree_pre=1, ratio=6.0, cycles=3, smooth=True, pin=True), "level", True, "cta"),
     ("nosell193-quad", 192, "quadrilateral", {"HEMO_SELL": "0", "HEMO_PDL": "0"},
      dict(degree=2, degree_pre=1, ratio=4.0, cycles=1, smooth=False), "level", False, "cta"),
-    ("nofuse41", 40, "triangle", {"HEMO_FUSE_MAX": "1"},
-     dict(degree=2, degree_pre=2, ratio=6.0, cycles=3, smooth=True), "level", False, "dense"),
-    ("fused41-top", 40, "triangle", {"HEMO_FUSE_MAX": "4000"},
-     dict(degree=3, degree_pre=1, ratio=4.0, cycles=3, smooth=True), "cta", False, "cta"),
     ("fused15-nc3", 14, "triangle", {}, dict(degree=2, degree_pre=1, ratio=6.0, cycles=3, smooth=False),
      "cta", False, "cta"),
     ("fused15-nc1-nopdl", 14, "quadrilateral", {"HEMO_PDL": "0", "HEMO_NO_GRAPH": "1"},
@@ -222,20 +217,6 @@ def test_amg_matches_oracle(monkeypatch, case):
             _check_coarse_shift(c, tag)
         print(f"AMGREF {tag:<22s} prolongation {_prolongation_kernel(c, 0)} (velocity), "
               f"{_prolongation_kernel(c, 1)} (pressure)")
-    finally:
-        c["hemo"].close()
-
-
-@pytest.mark.parametrize("env,scope", [({"HEMO_NO_GRAPH": "1", "HEMO_GRID_FUSE_MAX": "100000"}, "grid"),
-                                       ({"HEMO_CLUSTER_FUSE_MAX": "100000"}, "cluster")], ids=["grid", "cluster"])
-def test_amg_fused_grid_and_cluster(monkeypatch, env, scope):
-    """The cooperative-grid and thread-block-cluster fused kernels (off by default) where this GPU can run them."""
-    c = _lid_case(monkeypatch, 192, "triangle", env, degree=2, degree_pre=1, ratio=4.0, cycles=3, smooth=True)
-    try:
-        for which in (0, 1):
-            info = _check_apply(c, scope, which)
-            if not any(d["scope"] == scope for d in info):
-                pytest.skip(f"the {scope} fused kernel did not run here: {info}")
     finally:
         c["hemo"].close()
 

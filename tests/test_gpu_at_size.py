@@ -66,7 +66,7 @@ def test_one_million_cell_linear_solve_residual():
     s = sc.solver
     s._residual(s.d_x, s.d_f)
     s.hemo.assemble_jacobian(s.d_x, s.d_un, s.d_vals)
-    s.linear.setup(s.d_vals, s.d_x, s.d_un)
+    s.linear.setup(s.d_vals)
     its, rel = s.linear.solve(s.d_vals, s.d_f, s.d_y)
     assert 0 < its < 200 and rel <= 1e-9
     s.hemo.spmv(s.d_vals, s.d_y, s.d_w)

@@ -295,7 +295,7 @@ def test_tet_schur_operators_and_loud_failures():
     exact = (1 / 3 + 4 / 3 + 1.0) + 1 / 3 + 1.0
     assert abs(hemo.l2_norm_sq(T(u), 3) - exact) < 1e-12
     assert abs(hemo.l2_norm_sq(T(np.full(n, 2.0)), 1) - 4.0) < 1e-12
-    # the drag / lift integrals are the 2-D DFG forms; the assembled Schur operator is triangles-only
+    # the drag / lift integrals are the 2-D DFG forms
     with pytest.raises(HemoError):
         hemo.boundary_force(0, T(np.zeros(4 * n)))
     with pytest.raises(HemoError):

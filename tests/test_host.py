@@ -124,6 +124,20 @@ def test_no_gpu_is_a_loud_failure(hemo_lib_built):
         _lib.Hemo(0)
 
 
+def test_block_schur_solver_rejects_unknown_schur_mode():
+    """A Schur approximation the library does not implement is refused before the library is touched."""
+    from cfd_hemodynamic_b200.linear_solver import BlockSchurSolver
+
+    class NoLibrary:
+        def __getattr__(self, name):
+            raise AssertionError(f"library call {name} before the schur_mode check")
+
+    nrowptr, ncol = D.node_graph(np.array([[0, 1, 2]]), 3)
+    none = np.zeros(0, dtype=np.int64)
+    with pytest.raises(ValueError, match="schur_mode"):
+        BlockSchurSolver(NoLibrary(), nrowptr, ncol, none, none, dt=0.01, rho=1.0, mu=0.01, schur_mode="assembled")
+
+
 def test_amg_transfer_operators(hemo_lib_built):
     from cfd_hemodynamic_b200.fem import amg_setup
     m = M.create_unit_square(None, 24, 24)

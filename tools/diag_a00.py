@@ -6,7 +6,7 @@ with contextlib.redirect_stdout(sys.stderr):
 s = sc.solver
 for i in range(3): s.step_device()
 h = s.hemo; n = s.n
-h.assemble_jacobian(s.d_x, s.d_un, s.d_vals); s.linear.setup(s.d_vals, s.d_x, s.d_un)
+h.assemble_jacobian(s.d_x, s.d_un, s.d_vals); s.linear.setup(s.d_vals)
 rowptr, col = h.get_pattern()
 A = sp.csr_matrix((s.d_vals.cpu().numpy(), col.cpu().numpy(), rowptr.cpu().numpy()), shape=(3*n, 3*n))
 A00 = A[:2*n, :2*n].tocsr(); A11 = A[2*n:, 2*n:].tocsr(); A01 = A[:2*n, 2*n:].tocsr(); A10 = A[2*n:, :2*n].tocsr()
