@@ -27,7 +27,10 @@ class HemoError(RuntimeError):
 
 
 class HemoDiverged(HemoError):
-    pass
+    """A solve that ended without converging.  `Hemo.fgmres` attaches the iteration count (`its`) and the relative
+    residual estimate (`rel_resid`) of the iterate it has written; other callers leave them None."""
+    its = None
+    rel_resid = None
 
 
 class Params(C.Structure):
@@ -534,5 +537,9 @@ class Hemo:
         its = C.c_int()
         res = C.c_double()
         rc = self.lib.hemo_fgmres(self._ctx, _ptr(vals), _ptr(b), _ptr(y), C.byref(its), C.byref(res))
-        self._check(rc, "hemo_fgmres")
+        try:
+            self._check(rc, "hemo_fgmres")
+        except HemoDiverged as e:
+            e.its, e.rel_resid = its.value, res.value
+            raise
         return its.value, res.value

@@ -7,7 +7,8 @@
 // residual estimate and the convergence flag are updated by the last block of the update kernel; every kernel reads
 // the column index j from the device state, so the arguments of one iteration never change and the iteration
 // (preconditioner + SpMV + multi-dot + multi-axpy/norm/Givens) replays as ONE CUDA graph.  The host only polls the
-// state at the iteration count it expects from the previous solve; kernels queued beyond convergence exit at once.
+// state at the iteration count it expects from the previous solve; the k_fg_* kernels queued beyond convergence exit at
+// once (the preconditioner's kernels run again on the stale input, and nothing reads their output).
 //
 // Basis vectors are stored unnormalised with their scale s_j = 1/||w_j|| (device array): the SpMV writes w straight
 // into slot j+1, the update kernel orthogonalises it in place, and the "normalise" pass of textbook GMRES disappears
@@ -105,7 +106,8 @@ __global__ void k_fg_begin_cycle(FgState* st, const double* __restrict__ normsq,
                                  double* __restrict__ g, double* __restrict__ scale, int m) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
     if (!first && st->converged) return;
-    const double beta = sqrt(fmax(normsq[0], 0.0));
+    // a sum of squares: no fmax clamp, which would turn a NaN (a non-finite entry) into a zero norm
+    const double beta = sqrt(normsq[0]);
     if (first) {
         st->its = 0;
         st->converged = 0;
@@ -331,7 +333,7 @@ __device__ void fg_givens(FgState* st, int m, const double* __restrict__ hcol, d
         st->res = res;
         st->its += 1;
         scale[j + 1] = hn > 0.0 ? 1.0 / hn : 0.0;
-        if (!isfinite(res)) st->converged = -1;
+        if (!isfinite(res) || !isfinite(d)) st->converged = -1;     // d: a non-finite column gives c = 1, s = 0
         else if (res <= st->tol) st->converged = 1;
         else if (hn == 0.0) st->converged = 2;
         if (j + 1 >= m) st->cycle_full = 1;
@@ -376,7 +378,7 @@ k_fg_maxpy(FgState* st, FgSeg seg, int64_t nloc, double* __restrict__ V, int64_t
         total = s;
     }
     __syncthreads();
-    if (do_givens) fg_givens(st, m, hcol, sqrt(fmax(total, 0.0)), H, cs, sn, g, scale, hsh);
+    if (do_givens) fg_givens(st, m, hcol, sqrt(total), H, cs, sn, g, scale, hsh);
 }
 
 // multi-GPU: Givens after the norm has been summed over the ranks
@@ -387,7 +389,7 @@ __global__ void k_fg_givens(FgState* st, int m, const double* __restrict__ hcol,
     hemo_pdl_wait();
     hemo_pdl_trigger();
     if (st->converged || st->cycle_full) return;
-    fg_givens(st, m, hcol, sqrt(fmax(normsq[0], 0.0)), H, cs, sn, g, scale, gsh);
+    fg_givens(st, m, hcol, sqrt(normsq[0]), H, cs, sn, g, scale, gsh);
 }
 
 // ---- end of a cycle: y += Z_k (H_k^-1 g_k) ------------------------------------------------------------------------

@@ -137,3 +137,67 @@ def oracle_problem_from_solver(s, facet_tags=None, tags=None):
                              beta_b=s.beta_backflow))
     prob.facet_sets = fs
     return prob
+
+
+def lid_case(monkeypatch, nx, cell="triangle", env=None, *, pin=False, smooth=True, degree=2, degree_pre=1, ratio=4.0,
+             cycles=1, oracle=True):
+    """Fresh context with the lid-cavity Jacobian and a set-up block preconditioner (walls and lid: Dirichlet
+    multiplicity 2 at the top corners).  `env` is set before the context is created; `oracle` adds the float64 AMG
+    models of both hierarchies (oracle/amg_oracle.py) as "Hu" and "Hp"."""
+    import scipy.sparse as sp
+    import torch
+    from cfd_hemodynamic_b200._lib import Hemo
+    from cfd_hemodynamic_b200.linear_solver import BlockSchurSolver
+    from oracle import amg_oracle as AO
+    for k, v in (env or {}).items():
+        monkeypatch.setenv(k, v)
+    hemo = Hemo(0)
+    mesh = M.create_unit_square(None, nx, nx, cell_type=cell)
+    prob = make_problem(mesh, dt=0.01, rho=1.0, mu=0.05, f=(0.0, 0.0))
+    x, n = prob.x, prob.n
+    ext = M.exterior_facet_indices(mesh.topology)
+    walls = np.nonzero(np.isclose(x[:, 0], 0) | np.isclose(x[:, 0], 1) | np.isclose(x[:, 1], 0))[0]
+    lidf = M.locate_entities_boundary(mesh, 1, lambda X: np.isclose(X[1], 1.0) & (X[0] > 1e-10) & (X[0] < 1 - 1e-10))
+    lid = np.unique(mesh.topology.facet_vertices[lidf])
+    g1 = np.zeros(2 * n)
+    g1[0::2] = 1.0
+    bcs = [("u", walls, np.zeros(2 * n)), ("u", lid, g1)]
+    pnodes = np.zeros(0, dtype=np.int64)
+    if pin:                                   # one pinned pressure dof in the middle of the bottom wall
+        pnodes = np.array([int(np.argmin(np.abs(x[:, 0] - 0.5) + np.abs(x[:, 1])))])
+        bcs.append(("p", pnodes, np.zeros(n)))
+    prob.facet_sets = [O.FacetSet(pairs=mesh.topology.facet_cell_pairs(ext), a_p=1.0, a_g=1.0)]
+    _, (nrowptr, ncol) = setup_gpu(hemo, mesh, prob, [(ext, dict(a_p=1.0, a_g=1.0))], bcs)
+    u, p, un = smooth_fields(x, seed=2, U=0.5)
+    vals = torch.zeros(hemo.nnz, dtype=torch.float64, device=hemo.device)
+    hemo.assemble_jacobian(torch.tensor(np.concatenate([u, p]), device=hemo.device),
+                           torch.tensor(un, device=hemo.device), vals)
+    rowptr, col = hemo.get_pattern()
+    J = sp.csr_matrix((vals.cpu().numpy(), col.cpu().numpy(), rowptr.cpu().numpy()), shape=(3 * n, 3 * n))
+    s = BlockSchurSolver(hemo, nrowptr, ncol, np.unique(np.concatenate([walls, lid])), pnodes, dt=prob.dt, rho=prob.rho,
+                         mu=prob.mu, project_pressure=not pin, smooth_prolongator=smooth, cheb_degree=degree,
+                         cheb_degree_pre=degree_pre, cheb_ratio=ratio, amg_cycles_u=cycles, amg_cycles_p=cycles)
+    s.setup(vals)
+    pflag = np.zeros(n, dtype=bool)
+    pflag[pnodes] = True
+    lap = sp.csr_matrix((s.lap.cpu().numpy(), ncol, nrowptr), shape=(n, n))
+    c = dict(hemo=hemo, s=s, n=n, nx=nx, J=J, vals=vals, nrowptr=nrowptr, ncol=ncol, lap=lap, pflag=pflag, pin=pin,
+             project=not pin, cycles=cycles, kw=dict(degree=degree, degree_pre=degree_pre, ratio=ratio))
+    if oracle:
+        c["Hp"] = AO.Hierarchy(AO.pressure_level0(lap, pflag), s.levels[1], 1, 0.0 if pin else 1e-8)
+        c["Hu"] = velocity_oracle(c)
+    return c
+
+
+def velocity_oracle(c, mask=None):
+    """The float64 model of the velocity hierarchy of a `lid_case`, with the preconditioner's node mask."""
+    from oracle import amg_oracle as AO
+    return AO.Hierarchy(AO.velocity_level0(c["J"], c["n"], mask), c["s"].levels[0], 2)
+
+
+def amg_paths(c, which):
+    """amg_level_info of every level of hierarchy `which` of a `lid_case`, and the levels inside the fused coarse
+    V-cycle kernel."""
+    h = c["hemo"]
+    info = [h.amg_level_info(which, l) for l in range(len(c["s"].levels[which]) + 1)]
+    return info, {l for l, d in enumerate(info) if d["scope"] == "cta"}

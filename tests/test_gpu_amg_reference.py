@@ -26,63 +26,6 @@ TOL = AO.AMG_TOL
 GALERKIN_TOL = 1e-6       # level operators: the same float32-rounded products, summed in a different order
 
 
-def _lid_case(monkeypatch, nx, cell="triangle", env=None, *, pin=False, smooth=True, degree=2, degree_pre=1, ratio=4.0,
-              cycles=1):
-    """Fresh context with the lid-cavity Jacobian and a set-up block preconditioner."""
-    from cfd_hemodynamic_b200._lib import Hemo
-    from cfd_hemodynamic_b200.fem import mesh as M
-    from cfd_hemodynamic_b200.linear_solver import BlockSchurSolver
-    from oracle import ns_oracle as O
-    for k, v in (env or {}).items():
-        monkeypatch.setenv(k, v)
-    hemo = Hemo(0)
-    mesh = M.create_unit_square(None, nx, nx, cell_type=cell)
-    prob = T.make_problem(mesh, dt=0.01, rho=1.0, mu=0.05, f=(0.0, 0.0))
-    x, n = prob.x, prob.n
-    ext = M.exterior_facet_indices(mesh.topology)
-    walls = np.nonzero(np.isclose(x[:, 0], 0) | np.isclose(x[:, 0], 1) | np.isclose(x[:, 1], 0))[0]
-    lidf = M.locate_entities_boundary(mesh, 1, lambda X: np.isclose(X[1], 1.0) & (X[0] > 1e-10) & (X[0] < 1 - 1e-10))
-    lid = np.unique(mesh.topology.facet_vertices[lidf])
-    g1 = np.zeros(2 * n)
-    g1[0::2] = 1.0
-    bcs = [("u", walls, np.zeros(2 * n)), ("u", lid, g1)]
-    pnodes = np.zeros(0, dtype=np.int64)
-    if pin:                                   # one pinned pressure dof in the middle of the bottom wall
-        pnodes = np.array([int(np.argmin(np.abs(x[:, 0] - 0.5) + np.abs(x[:, 1])))])
-        bcs.append(("p", pnodes, np.zeros(n)))
-    prob.facet_sets = [O.FacetSet(pairs=mesh.topology.facet_cell_pairs(ext), a_p=1.0, a_g=1.0)]
-    _, (nrowptr, ncol) = T.setup_gpu(hemo, mesh, prob, [(ext, dict(a_p=1.0, a_g=1.0))], bcs)
-    u, p, un = T.smooth_fields(x, seed=2, U=0.5)
-    vals = torch.zeros(hemo.nnz, dtype=torch.float64, device=hemo.device)
-    hemo.assemble_jacobian(torch.tensor(np.concatenate([u, p]), device=hemo.device),
-                           torch.tensor(un, device=hemo.device), vals)
-    rowptr, col = hemo.get_pattern()
-    J = sp.csr_matrix((vals.cpu().numpy(), col.cpu().numpy(), rowptr.cpu().numpy()), shape=(3 * n, 3 * n))
-    s = BlockSchurSolver(hemo, nrowptr, ncol, np.unique(np.concatenate([walls, lid])), pnodes, dt=prob.dt, rho=prob.rho,
-                         mu=prob.mu, project_pressure=not pin, smooth_prolongator=smooth, cheb_degree=degree,
-                         cheb_degree_pre=degree_pre, cheb_ratio=ratio, amg_cycles_u=cycles, amg_cycles_p=cycles)
-    s.setup(vals)
-    pflag = np.zeros(n, dtype=bool)
-    pflag[pnodes] = True
-    lap = sp.csr_matrix((s.lap.cpu().numpy(), ncol, nrowptr), shape=(n, n))
-    c = dict(hemo=hemo, s=s, n=n, J=J, vals=vals, nrowptr=nrowptr, ncol=ncol, lap=lap, pflag=pflag, pin=pin,
-             project=not pin, cycles=cycles, kw=dict(degree=degree, degree_pre=degree_pre, ratio=ratio))
-    c["Hp"] = AO.Hierarchy(AO.pressure_level0(lap, pflag), s.levels[1], 1, 0.0 if pin else 1e-8)
-    c["Hu"] = _velocity_oracle(c)
-    return c
-
-
-def _velocity_oracle(c, mask=None):
-    return AO.Hierarchy(AO.velocity_level0(c["J"], c["n"], mask), c["s"].levels[0], 2)
-
-
-def _paths(c, which):
-    """amg_level_info of every level, and the levels inside the fused coarse V-cycle kernel."""
-    h = c["hemo"]
-    info = [h.amg_level_info(which, l) for l in range(len(c["s"].levels[which]) + 1)]
-    return info, {l for l, d in enumerate(info) if d["scope"] == "cta"}
-
-
 def _prolongation_kernel(c, which):
     """Kernel of the top-level prolongation (the rule of vcycle_t)."""
     P, n = c["s"].levels[which][0]["P"], c["n"]
@@ -116,7 +59,7 @@ def _check_galerkin(c, tag):
 def _check_apply(c, tag, which, seed=0, note=""):
     h, n = c["hemo"], c["n"]
     H = c["Hu"] if which == 0 else c["Hp"]
-    info, fused = _paths(c, which)
+    info, fused = T.amg_paths(c, which)
     rng = np.random.default_rng(seed + which)
     b = rng.standard_normal(H.ops[0].shape[0])
     singular = which == 1 and c["project"]
@@ -144,13 +87,13 @@ def _check_coarse_shift(c, tag, shift=0.25):
 
 def _check_pc(c, tag, mask=None, seed=5):
     h, n, s = c["hemo"], c["n"], c["s"]
-    _, fused_u = _paths(c, 0)
-    _, fused_p = _paths(c, 1)
+    _, fused_u = T.amg_paths(c, 0)
+    _, fused_p = T.amg_paths(c, 1)
     Hu = c["Hu"]
     if mask is not None:
         h.set_pc_mask(torch.tensor(mask.astype(np.uint8), device=h.device))
         s.setup(c["vals"])
-        Hu = _velocity_oracle(c, mask)
+        Hu = T.velocity_oracle(c, mask)
     try:
         rng = np.random.default_rng(seed)
         r = rng.standard_normal(3 * n)
@@ -197,7 +140,7 @@ CASES = [
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
 def test_amg_matches_oracle(monkeypatch, case):
     tag, nx, cell, env, opts, scope0, sell0, scope_last = case
-    c = _lid_case(monkeypatch, nx, cell, env, **opts)
+    c = T.lid_case(monkeypatch, nx, cell, env, **opts)
     try:
         _check_galerkin(c, tag)
         for which in (0, 1):
@@ -225,7 +168,7 @@ def test_solver_opts_take_effect_without_new_setup(monkeypatch):
     """Changing options between calls (no new hemo_pc_setup) reaches the captured graphs of hemo_amg_apply,
     hemo_pc_apply and the FGMRES iteration."""
     tag = "stale-opts41"
-    c = _lid_case(monkeypatch, 40, "triangle", {}, degree=2, degree_pre=1, ratio=4.0, cycles=1)
+    c = T.lid_case(monkeypatch, 40, "triangle", {}, degree=2, degree_pre=1, ratio=4.0, cycles=1)
     h, s, n = c["hemo"], c["s"], c["n"]
     try:
         rng = np.random.default_rng(11)
@@ -246,8 +189,8 @@ def test_solver_opts_take_effect_without_new_setup(monkeypatch):
         h.amg_apply(0, bd, xd, 1)
         _report(tag, "amg_apply degree 3, same buffers", AO.rel_errors(xd.cpu().numpy(), c["Hu"].apply(b, 1, **kw)))
         h.pc_apply(c["vals"], r, z)
-        _, fused_u = _paths(c, 0)
-        _, fused_p = _paths(c, 1)
+        _, fused_u = T.amg_paths(c, 0)
+        _, fused_p = T.amg_paths(c, 1)
         ref = AO.pc_apply_laplace(r.cpu().numpy(), n, c["Hu"], c["Hp"], AO.a01_block(c["J"], n), s.mass.cpu().numpy(),
                                   mass_coef=s.opts["schur_mass_coef"], lap_coef=s.opts["schur_lap_coef"],
                                   project_pressure=True, cycle_kw_u=dict(fused=fused_u, **kw),
@@ -258,7 +201,7 @@ def test_solver_opts_take_effect_without_new_setup(monkeypatch):
     finally:
         h.close()
     # the same solve in a context that had degree 3 from the start
-    f = _lid_case(monkeypatch, 40, "triangle", {}, degree=3, degree_pre=1, ratio=4.0, cycles=1)
+    f = T.lid_case(monkeypatch, 40, "triangle", {}, degree=3, degree_pre=1, ratio=4.0, cycles=1)
     try:
         yf = torch.zeros(3 * n, dtype=torch.float64, device=f["hemo"].device)
         its3_fresh, _ = f["s"].solve(f["vals"], rhs, yf)
